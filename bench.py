@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- stereo pairs/sec for GwcNet @256x512, D=192 (BASELINE.json metric), 1..8 x B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 8]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--batch 8] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one GwcNet inference forward (2D backbone -> cost volume -> 3D aggregation -> soft-argmin) over one batch
@@ -24,6 +24,11 @@ Reported in one JSON line (rank 0):
   comparators  the unmodified reference on the same B200 (cuDNN fp32, TF32 off) and its Triton gwc kernel
                (fast_foundationstereo/core/submodule.py:443-478) against this library's gwc volume kernel
 --impl reference times the reference's own CPU implementation as the reference arm.
+--dump-outputs DIR writes what the last timed step returned (rank 0) as float32 .npy files: disp_pred.npy, the (B, 256, 512)
+disparities of that step's batch, and epe_partials.npy, the gathered (B * n_gpus, 2) per-image {sum |err|, #valid}
+(--impl reference: disp_pred.npy of its 1-pair step).  Inputs and weights are seeded, so two builds run with the same
+arguments can be compared output for output.  The EPE sums are float32 block partials added with atomics, so they vary
+in the last bits from run to run; disp_pred does not.
 """
 import argparse
 import json
@@ -224,7 +229,9 @@ def run_reference(args):
     torch.set_num_threads(cores)
     model, kind = reference_model()
     pairs = 1                                                       # bounded sample: one pair of the B=8 batch per step
-    dt, _ = time_cpu(model, pairs, args.steps, min(args.warmup, 2))
+    dt, out = time_cpu(model, pairs, args.steps, min(args.warmup, 2))
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"disp_pred": out})
     value = pairs * args.steps / dt
     line = {
         "impl": "reference", "metric": METRIC, "value": value, "unit": "pairs/s", "n_gpus": args.gpus, "steps": args.steps,
@@ -266,7 +273,7 @@ def run_ours(args):
         k = i % rot
         with torch.no_grad():
             disp = model({"left": dev_left[k], "right": dev_right[k]})["disp_pred"]
-            return ops.epe_partial(disp, dev_gt[k], CFG["MAX_DISP"])
+            return disp, ops.epe_partial(disp, dev_gt[k], CFG["MAX_DISP"])
 
     def step_e2e(i):
         k = i % rot
@@ -278,7 +285,7 @@ def run_ours(args):
             part = ops.epe_partial(disp, gt, CFG["MAX_DISP"])
             host_epe.copy_(part, non_blocking=True)
             torch.cuda.current_stream().synchronize()               # the caller reads the metric every step
-            return part
+            return disp, part
 
     from openstereo_b200.distributed import gather_epe_partials
 
@@ -293,9 +300,9 @@ def run_ours(args):
         launches0 = _lib.launch_count()
         start, stop = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         start.record()
-        part = None
+        disp = part = None
         for i in range(steps):
-            part = step_fn(i)
+            disp, part = step_fn(i)
         allparts = gather(part)
         stop.record()
         torch.cuda.synchronize()
@@ -311,7 +318,7 @@ def run_ours(args):
             sm = t.clone()
             dist.all_reduce(sm, op=dist.ReduceOp.SUM)
             ms, launches = mx[0].item(), int(sm[1].item())
-        return ms, launches, prof, allparts
+        return ms, launches, prof, allparts, disp
 
     for i in range(max(args.warmup, 3)):
         step_resident(i)
@@ -323,10 +330,13 @@ def run_ours(args):
         sampler.start()
     if os.environ.get("OSB_NCU_RANGE"):                             # `ncu --profile-from-start off`: capture only the timed steps
         torch.cuda.cudart().cudaProfilerStart()
-    ms, launches, prof, parts = timed(step_resident, args.steps, profile=True)
+    ms, launches, prof, parts, last_disp = timed(step_resident, args.steps, profile=True)
     if os.environ.get("OSB_NCU_RANGE"):
         torch.cuda.cudart().cudaProfilerStop()
-    ms_e2e, _, _, _ = timed(step_e2e, args.steps, profile=False)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"disp_pred": last_disp, "epe_partials": parts})
+    del last_disp
+    ms_e2e, _, _, _, _ = timed(step_e2e, args.steps, profile=False)
     clocks = sampler.stop(args.gpus) if rank == 0 else None
     if rank != 0:
         if world > 1:
@@ -463,6 +473,14 @@ def run_ours(args):
         dist.destroy_process_group()
 
 
+def dump_outputs(path, arrays):
+    """name -> tensor, written as path/<name>.npy in float32."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), t.detach().float().cpu().numpy())
+
+
 def run_comparators(args, dev, B, dev_left, dev_right, dev_gt, mirror_value):
     """N = 1 legs that need the staged reference (oracle/_ref).  Each is CUDA-event timed after warm-up, resident inputs, same
     synthetic weights and batches as the main arm.
@@ -549,7 +567,11 @@ def main():
     ap.add_argument("--rotate", type=int, default=12)
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-comparators", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the last timed step's outputs as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         run_reference(args)
     else:

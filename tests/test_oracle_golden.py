@@ -1,5 +1,10 @@
 """CPU: the oracle restatement reproduces the reference's own outputs (tests/golden/*.npz,
-written by tools/make_golden.py from the unmodified reference) BIT-EXACTLY."""
+written by tools/make_golden.py from the unmodified reference) BIT-EXACTLY.
+
+Exception: outputs of CPU kernels whose summation order depends on the host CPU -- 3D/2D convolutions, the geometry
+lookup's batched matmul, trilinear interpolation, the per-image EPE mean -- agree with vectors stored on another host to
+within fp32 reordering, REORDER of the output's largest magnitude (assert_reordered); on the host that wrote them they
+are bit-equal."""
 import pytest
 import torch
 
@@ -11,6 +16,14 @@ from oracle import regression as oreg
 from oracle import seeded_init as si
 
 from conftest import load_golden
+
+
+REORDER = 1e-5
+
+
+def assert_reordered(got, want):
+    assert got.shape == want.shape
+    assert (got - want).abs().max().item() <= REORDER * want.abs().max().item()
 
 
 def checksum(sd):
@@ -55,12 +68,12 @@ def test_regression_tails():
     with pytest.raises(ValueError):
         oreg.faster_soft_argmin(g["cost"][0], g["maxdisp"])
     g = load_golden("upsample_softargmin")
-    assert torch.equal(oreg.upsample_softargmin(g["cost"], g["maxdisp"], g["out_h"], g["out_w"]), g["out_gwc"])
-    assert torch.equal(oreg.upsample_softargmin(g["cost"], g["maxdisp"], g["out_h"], g["out_w"], align_corners=True,
-                                                psm_tail=True), g["out_psm"])
+    assert_reordered(oreg.upsample_softargmin(g["cost"], g["maxdisp"], g["out_h"], g["out_w"]), g["out_gwc"])
+    assert_reordered(oreg.upsample_softargmin(g["cost"], g["maxdisp"], g["out_h"], g["out_w"], align_corners=True,
+                                              psm_tail=True), g["out_psm"])
     g = load_golden("epe_per_image")
     mask = (g["gt"] < 192) & (g["gt"] > 0)
-    assert torch.equal(oreg.epe_per_image(g["pred"], g["gt"], mask), g["out"])
+    assert_reordered(oreg.epe_per_image(g["pred"], g["gt"], mask), g["out"])
 
 
 def test_modules():
@@ -70,19 +83,20 @@ def test_modules():
         sd = si.seeded_state_dict(m.state_dict(), seed=g["seed"])
         assert checksum(sd) == pytest.approx(g["sd_checksum"], rel=1e-12)
         m.load_state_dict(sd)
-        assert torch.equal(m(g["x"]), g["out"])
+        assert_reordered(m(g["x"]), g["out"])
 
         g = load_golden("gwc_disp_processor")
         m = oagg.GwcDispProcessor(maxdisp=32, downsample=4, num_groups=4, use_concat_volume=True, concat_channels=2).eval()
         m.load_state_dict(si.seeded_state_dict(m.state_dict(), seed=g["seed"], scale={"classif3.2.weight": 60.0}))
-        assert torch.equal(m(g["volume"], 32, 64), g["out"])
+        assert_reordered(m(g["volume"], 32, 64), g["out"])
 
         g = load_golden("psm_aggregator")
         m = oagg.PSMAggregator(32, 8).eval()
         m.load_state_dict(si.seeded_state_dict(m.state_dict(), seed=g["seed"], scale={
             "classif1.1.weight": 20.0, "classif2.1.weight": 20.0, "classif3.1.weight": 20.0}))
         low = m.aggregate(g["raw"])
-        assert torch.equal(low[2], g["cost3_low"]) and torch.equal(low[0], g["cost1_low"])
+        assert_reordered(low[2], g["cost3_low"])
+        assert_reordered(low[0], g["cost1_low"])
 
         g = load_golden("stereobase_head")
         m = oagg.StereoBaseCostHead(8, [16, 16, 24, 20], max_disp=64).eval()
@@ -91,7 +105,8 @@ def test_modules():
         sd.update({"cost_agg." + k: v for k, v in sd_h.items()})
         m.load_state_dict(sd)
         geo, init_disp = m(g["volume"], [g["f0"], g["f1"], g["f2"], g["f3"]])
-        assert torch.equal(geo, g["geo"]) and torch.equal(init_disp, g["init_disp"])
+        assert_reordered(geo, g["geo"])
+        assert_reordered(init_disp, g["init_disp"])
 
 
 def test_gwcnet_model():
@@ -102,7 +117,7 @@ def test_gwcnet_model():
     m.load_state_dict(sd)
     with torch.no_grad():
         out = m({"left": g["left"], "right": g["right"]})["disp_pred"]
-    assert torch.equal(out, g["out"])
+    assert_reordered(out, g["out"])
     assert out.std() > 10.0          # the seeded init is not the degenerate constant-95.5 case
 
 
@@ -112,22 +127,23 @@ def test_psmnet_model():
     m.load_state_dict(si.seeded_state_dict(m.state_dict(), seed=g["seed"], scale=si.PSMNET_SCALE, keep=si.PSMNET_KEEP))
     with torch.no_grad():
         out = m({"left": g["left"], "right": g["right"]})["disp_pred"]
-    assert torch.equal(out, g["out"])
+    assert_reordered(out, g["out"])
 
 
 @pytest.mark.parametrize("name", ["geo_lookup_small", "geo_lookup_3lvl"])
 def test_geo_lookup(name):
-    """SURVEY.md section 8(f) row 1: the oracle reproduces the reference's lookup output and pyramid bit for bit."""
+    """SURVEY.md section 8(f) row 1: the oracle reproduces the reference's lookup output and pyramids."""
     g = load_golden(name)
     vol = ogeo.GeoEncodingVolume(g["fmap1"], g["fmap2"], g["volume"], num_levels=g["levels"], radius=g["radius"])
-    assert torch.equal(vol(g["disp"], g["coords"]), g["out"])
-    assert torch.equal(vol.geo_pyramid[-1], g["geo_last"]) and torch.equal(vol.corr_pyramid[-1], g["corr_last"])
+    assert_reordered(vol(g["disp"], g["coords"]), g["out"])
+    assert torch.equal(vol.geo_pyramid[-1], g["geo_last"])                        # pooling only: bit for bit
+    assert_reordered(vol.corr_pyramid[-1], g["corr_last"])
     assert g["out"].shape[1] == g["levels"] * (g["volume"].shape[1] + 1) * (2 * g["radius"] + 1)
 
 
 def test_context_upsample():
     g = load_golden("context_upsample")
-    assert torch.equal(ogeo.context_upsample(g["disp_low"], g["up_weights"], g["scale"]), g["out"])
+    assert_reordered(ogeo.context_upsample(g["disp_low"], g["up_weights"], g["scale"]), g["out"])
 
 
 def test_row4_volume_and_regression_flavours():
@@ -158,4 +174,5 @@ def test_lightstereo_aggregation():
     m.load_state_dict(sd)
     with torch.no_grad():
         out = m(g["x"], [g["f0"], g["f1"], g["f2"]])[0]
-    assert torch.equal(out, g["out"]) and out.std() > 1e-3
+    assert_reordered(out, g["out"])
+    assert out.std() > 1e-3

@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Generate tests/golden/*.npz by running the UNMODIFIED reference (authoring container only).
 
-    python tools/make_golden.py            # needs /root/reference
+    python tools/make_golden.py [group ...]     # needs the reference tree (oracle/_reference_shim.py); groups: GROUPS below
 
 For every case: seeded inputs -> the reference's own function/module (imported through
 oracle/_reference_shim.py) -> outputs saved next to the inputs.  While generating, the script also
@@ -304,15 +304,90 @@ def flavours():
     save("regression_flavours", prob=prob, maxdisp=48, interval=4, out_interval=ref, values=vals, out_values=ref2)
 
 
+def pinned(out, key, t, full_max=4096, n_sample=2048):
+    """Store a reference output under `key`: whole when it has at most `full_max` elements, otherwise a seeded sample of
+    `n_sample` elements (flat indices + values) with the shape and the float64 sum and absolute sum of the whole tensor."""
+    t = t.detach().contiguous()
+    if t.numel() <= full_max:
+        out[key] = t
+        return
+    idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(7))[:n_sample].sort().values
+    out[key + "__idx"], out[key + "__val"] = idx.int(), t.reshape(-1)[idx]
+    out[key + "__shape"] = torch.tensor(t.shape, dtype=torch.int64)
+    out[key + "__sum"], out[key + "__abssum"] = t.double().sum(), t.double().abs().sum()
+
+
+def pins():
+    """The reference outputs that tests/test_oracle_pins_reference.py, tests/test_patch_cpu.py and
+    tests/test_ops_gpu.py::test_sub_volume_vs_oracle_and_reference compare against, on the seeded inputs those tests
+    regenerate (same seeds, same shapes)."""
+    rcv = shim.load("stereo.modeling.cost_volume.cost_volume")
+    rpsm = shim.load("stereo.modeling.models.psmnet.psmnet_cost_processor")
+    rreg = shim.load("stereo.modeling.disp_pred.disp_regression")
+    rpdp = shim.load("stereo.modeling.models.psmnet.psmnet_disp_processor")
+    rgh = shim.load("stereo.modeling.models.gwcnet.hourglass")
+    rgeo = shim.load("stereo.modeling.models.igev.geometry")
+    rsb = shim.load("stereo.modeling.models.stereobase.gru_blocks")
+    rblk = shim.load("stereo.modeling.models.stereobase.igev_blocks")
+    out = {}
+    for b, c, h, w, d, g in [(2, 24, 4, 19, 7, 3), (1, 40, 3, 33, 40, 5), (1, 8, 2, 6, 9, 8)]:
+        tag = "%d_%d_%d_%d_%d_%d" % (b, c, h, w, d, g)
+        l, r = rnd(1, b, c, h, w), rnd(2, b, c, h, w)
+        pinned(out, "gwc_" + tag, rcv.build_gwc_volume(l, r, d, g))
+        concat = rcv.build_concat_volume(l, r, d)
+        must_equal(concat, rpsm.cat_fms(l, r, max_disp=d), "concat volume vs cat_fms " + tag)     # one array serves both
+        pinned(out, "concat_" + tag, concat)
+        pinned(out, "corr_" + tag, rcv.correlation_volume(l, r, d))
+    p = torch.softmax(rnd(3, 2, 20, 5, 6) * 3, 1)
+    out["regression"] = rreg.disparity_regression(p, 20)
+    out["faster_softargmin"] = rpdp.FasterSoftArgmin(max_disp=20, alpha=2.0)(rnd(4, 2, 20, 5, 6))
+    with torch.no_grad():
+        ref = rgh.Hourglass(8).eval()
+        ref.load_state_dict(si.seeded_state_dict(ref.state_dict(), seed=5))
+        x = rnd(6, 1, 8, 4, 8, 8)
+        out["gwc_hourglass"] = ref(x)
+        ref = rpsm.Hourglass(8).eval()
+        ref.load_state_dict(si.seeded_state_dict(ref.state_dict(), seed=7))
+        for i, t in enumerate(ref(x, rnd(8, 1, 16, 2, 4, 4), rnd(9, 1, 16, 2, 4, 4))):
+            out["psm_hourglass_%d" % i] = t
+    for b, cf, cg, d, h, w, levels, radius in [(1, 5, 8, 24, 4, 30, 2, 4), (2, 3, 2, 9, 2, 11, 1, 3)]:
+        f1, f2, vol = rnd(70, b, cf, h, w), rnd(71, b, cf, h, w), rnd(72, b, cg, d, h, w)
+        disp = torch.rand(b, 1, h, w, generator=torch.Generator().manual_seed(73)) * (d + 4) - 2
+        coords = torch.arange(w).float().reshape(1, 1, w, 1).repeat(b, h, 1, 1)
+        a = rgeo.Combined_Geo_Encoding_Volume(f1, f2, vol, num_levels=levels, radius=radius)(disp, coords)
+        must_equal(a, rsb.CombinedGeoEncodingVolume(f1, f2, vol, num_levels=levels, radius=radius)(disp, coords),
+                   "geo lookup: igev vs stereobase class")
+        pinned(out, "geo_%d_%d_%d_%d_%d_%d_%d_%d" % (b, cf, cg, d, h, w, levels, radius), a)
+    low, wts = rnd(74, 2, 1, 6, 9).abs() * 30, torch.softmax(rnd(75, 2, 9, 24, 36), dim=1)
+    out["context_upsample"] = rblk.context_upsample(low, wts)
+    save("pins_reference", **out)
+
+    # build_sub_volume allocates its output with device='cuda'; its arithmetic (an L1 norm over channels) is run here on
+    # the host by allocating that output on the inputs' device instead
+    zeros = torch.zeros
+    rcv.torch.zeros = lambda *a, device=None, **k: zeros(*a, **k)
+    try:
+        sub = {}
+        for shape, d in (((2, 12, 5, 37), 9), ((1, 96, 4, 128), 48), ((1, 3, 2, 6), 8)):
+            pinned(sub, "sub_%s_%d" % ("_".join(map(str, shape)), d), rcv.build_sub_volume(rnd(70, *shape), rnd(71, *shape), d))
+    finally:
+        rcv.torch.zeros = zeros
+    save("sub_volume_reference", **sub)
+
+    # the module globals StereoBase's forward and upsample_disp reach by name: what per-instance rebinding has to override
+    sbm = shim.load("stereo.modeling.models.stereobase.stereobase_gru")
+    names = (set(sbm.StereoBase.forward.__code__.co_names) | set(sbm.StereoBase.upsample_disp.__code__.co_names)) & set(vars(sbm))
+    save("stereobase_globals", names=np.array(sorted(names)))
+
+
+GROUPS = {"volumes": volumes, "regression": regression, "modules": modules, "models": models, "lookups": lookups,
+          "flavours": flavours, "lightstereo": lightstereo, "pins": pins}
+
+
 if __name__ == "__main__":
     if not shim.available():
-        raise SystemExit("reference tree not found; golden vectors can only be generated in the authoring container")
+        raise SystemExit("reference tree not found; golden vectors can only be generated where it is present")
     torch.set_num_threads(os.cpu_count() or 1)
-    volumes()
-    regression()
-    modules()
-    models()
-    lookups()
-    flavours()
-    lightstereo()
+    for name in sys.argv[1:] or GROUPS:
+        GROUPS[name]()
     print("all oracle restatements bit-equal to the reference; golden vectors written to", OUT)
