@@ -214,6 +214,39 @@ int osb_deconv3d_k4_tc_cs_fwd(const float* x_ndhwc, const void* w_split, const f
  * w_packed (C0+C1, Cout).  192 -> 96 and 128 -> 64. */
 int osb_conv1x1_ndhwc_cat_fwd(const float* x0, const float* x1, int C0, int C1, const float* w_packed, const float* scale,
                               const float* shift, float* y, long long voxels, int Cout, int act, osb_stream_t stream);
+/* ---- fp16 activations (suffix _h16): StereoBase's hourglass under torch.autocast(float16), opt-in (aggregation.StereoBaseAggregation
+ * precision="fp16", DESIGN.md section 4.11).  Same operators as the fp32 siblings above, with these differences:
+ *   - x / x0 / x1 and y hold fp16 values: inputs are `const void*`, the output keeps the ABI's `float*` spelling but receives
+ *     fp16 elements (2 bytes each); scale, shift and gate_nhwc stay fp32, w_split stays the fp16 pack;
+ *   - w_split is a hi-only pack (ops.pack_tc_weight(..., h16=True)): the lo halves of its rows are zero and never read, and
+ *     `scale` carries 2^-e_c times the folded-BN scale (no activation scale) -- every product is ONE kind::f16 MMA of fp16 operands;
+ *   - folded BN, activation and gate are applied in fp32, the result is stored with cvt.rn.satfinite: |y| > 65504 saturates and
+ *     increments the sticky counter of osb_tc_overflow_count / osb_tc_overflow_poll;
+ *   - channels-last x and y (deconv: NCDHW y with cout_real allowed when out_ndhwc = 0), no residual;
+ *   - shapes: the whole-row variants of StereoBase's hourglass at W' = 128, see the _h16_supported queries (W = input width):
+ *     stride 1: W=64/Cout=64, W=32/Cout=96, W=16/Cout=96|64 (channel slices); stride 2: W=128/Cout=64, W=64/Cout=96, W=32/Cout=96|64;
+ *     k4 transposed conv: osb_deconv3d_k4_tc_supported.  x, w_split and gate_nhwc 16-byte aligned, y 8-byte aligned. */
+int osb_conv3d_tc_h16_supported(int Cin, int Cout, int W);
+int osb_conv3d_s2_tc_h16_supported(int Cin, int Cout, int D, int H, int W);
+int osb_conv3d_k3_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                             int Cout, int D, int H, int W, int act, osb_stream_t stream);
+int osb_conv3d_k3_tc_gate_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, const float* gate_nhwc,
+                                  float* y, int B, int Cin, int Cout, int D, int H, int W, int act, osb_stream_t stream);
+int osb_conv3d_k3_s2_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                                int Cout, int D, int H, int W, int act, osb_stream_t stream);
+int osb_deconv3d_k4_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                               int Cout, int cout_real, int D, int H, int W, int act, int out_ndhwc, osb_stream_t stream);
+/* channel slices (see the _cs_fwd siblings); gate_nhwc (B,H,W,ystride) fp32 pre-offset to the slice, or NULL */
+int osb_conv3d_k3_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, const float* gate_nhwc,
+                                float* y, int B, int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream);
+int osb_conv3d_k3_s2_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                   int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream);
+int osb_deconv3d_k4_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                  int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream);
+/* osb_conv1x1_ndhwc_cat_fwd with fp16 slabs x0, x1 (8-byte aligned) and fp16 y; fp32 weights and arithmetic, saturating stores
+ * counted like the tensor-core convs'. */
+int osb_conv1x1_ndhwc_cat_h16_fwd(const void* x0, const void* x1, int C0, int C1, const float* w_packed, const float* scale,
+                                  const float* shift, float* y, long long voxels, int Cout, int act, osb_stream_t stream);
 /* Channels-last 1x1x1 conv + folded BN + activation (the redir branches when the aggregation runs channels-last):
  * x (voxels, Cin) -> y (voxels, Cout); w_packed (Cin, Cout).  32->32 and 64->64. */
 int osb_conv1x1_ndhwc_fwd(const float* x, const float* w_packed, const float* scale, const float* shift, float* y,
@@ -294,6 +327,8 @@ int osb_ncdhw_to_ndhwc(const float* x, float* y, int B, int C, int D, int H, int
 /* Same with the channel axis zero-padded to Cpad >= C: y (B,D,H,W,Cpad) -- channel plans that are not multiples of 16 (StereoBase's
  * 24 / 48) run on the tensor-core kernels as 32 / 64 with zero weights on the padding. */
 int osb_ncdhw_to_ndhwc_pad(const float* x, float* y, int B, int C, int Cpad, int D, int H, int W, osb_stream_t stream);
+/* Same for fp16 tensors: x (B,C,D,H,W) fp16 -> y (B,D,H,W,Cpad) fp16, padding zero. */
+int osb_ncdhw_to_ndhwc_pad_h16(const void* x, float* y, int B, int C, int Cpad, int D, int H, int W, osb_stream_t stream);
 /* FeatureAtt gate in one launch (igev_blocks.py:35-48 as used by stereobase/hourglass.py:62-99):
  * gate_nhwc (B,H,W,Cpad) = sigmoid(conv1x1(act1(bn(conv1x1(feat_nchw (B,Cf,H,W)))))), channels Cv..Cpad-1 zero.
  * w1_packed (Cf,Ch), w2_packed (Ch,Cv); scale/shift = folded BN / bias (NULL = identity).  HW = H*W. */

@@ -61,6 +61,17 @@ SIGNATURES = {
     "osb_softargmin_bwd": [_f32p] * 3 + [_i] * 4 + [_f, _f, _f, _i, _s],
     "osb_dwconv2d_fwd": [_f32p] * 6 + [_i] * 8 + [_s],
     "osb_deconv2d_k3s2_fwd": [_f32p] * 6 + [_i] * 6 + [_s],
+    "osb_conv3d_tc_h16_supported": [_i, _i, _i],
+    "osb_conv3d_s2_tc_h16_supported": [_i] * 5,
+    "osb_conv3d_k3_tc_h16_fwd": [_f32p] * 5 + [_i] * 7 + [_s],
+    "osb_conv3d_k3_tc_gate_h16_fwd": [_f32p] * 6 + [_i] * 7 + [_s],
+    "osb_conv3d_k3_s2_tc_h16_fwd": [_f32p] * 5 + [_i] * 7 + [_s],
+    "osb_deconv3d_k4_tc_h16_fwd": [_f32p] * 5 + [_i] * 9 + [_s],
+    "osb_conv3d_k3_tc_cs_h16_fwd": [_f32p] * 6 + [_i] * 8 + [_s],
+    "osb_conv3d_k3_s2_tc_cs_h16_fwd": [_f32p] * 5 + [_i] * 8 + [_s],
+    "osb_deconv3d_k4_tc_cs_h16_fwd": [_f32p] * 5 + [_i] * 8 + [_s],
+    "osb_conv1x1_ndhwc_cat_h16_fwd": [_f32p, _f32p, _i, _i, _f32p, _f32p, _f32p, _f32p, ctypes.c_longlong, _i, _i, _s],
+    "osb_ncdhw_to_ndhwc_pad_h16": [_f32p, _f32p, _i, _i, _i, _i, _i, _i, _s],
 }
 
 

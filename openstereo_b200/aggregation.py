@@ -159,10 +159,10 @@ class _Engine:
             self._stamp = stamp
 
     @staticmethod
-    def _check(x):
+    def _check(x, dtype=torch.float32):
         if not x.is_cuda:
             raise RuntimeError("openstereo_b200: not implemented on the CPU (no fallback); move the model to CUDA")
-        return x.detach().float().contiguous()
+        return x.detach().to(dtype).contiguous()
 
 
 # ------------------------------------------------------------------------------------------------------ GwcNet
@@ -403,7 +403,19 @@ def _block(m):
 
 
 class StereoBaseAggregation(_Engine):
-    """Hourglass(volume_channel, backbone_channels) with FeatureAtt gates: (B,C,D',H',W') + 2D features -> same shape."""
+    """Hourglass(volume_channel, backbone_channels) with FeatureAtt gates: (B,C,D',H',W') + 2D features -> same shape.
+
+    precision="fp32" (default): every input is computed with fp32-accurate products (3xFP16 split) and the result is fp32.
+    precision="fp16": a float16 volume (the model runs under torch.autocast(float16)) whose shape has the whole tensor-core route
+    (_h16_route_ok) stays fp16 end to end -- fp16 activations, one fp16 MMA per product, fp32 accumulation, BN / activation / gate
+    in fp32, fp16 stores that saturate at +-65504 and make the next call raise (ops.TcOverflowMonitor) -- and the result is fp16.
+    Any other input (fp32, bf16, other shapes) takes the fp32 path, as with precision="fp32"."""
+
+    def __init__(self, module, precision="fp32"):
+        if precision not in ("fp32", "fp16"):
+            raise ValueError("precision must be 'fp32' or 'fp16', got %r" % (precision,))
+        super().__init__(module)
+        self.precision = precision
 
     def _pack(self):
         m = self.module
@@ -445,10 +457,16 @@ class StereoBaseAggregation(_Engine):
                     and (2 * p4, p4) in ((192, 96), (128, 64)) and (2 * p2, p2) in ((192, 96), (128, 64))
                     and self.up["conv2_up"][0].kernel == 4 and self.up["conv1_up"][0].kernel == 4)
 
-    def _tc_pack(self):
-        """Zero-padded tensor-core packs of the layers on the 1/8 and 1/16 levels (built once per _ensure stamp)."""
-        if getattr(self, "_tcp_stamp", None) == self._stamp:
-            return self._tcp
+    def _tc_pack(self, h16=False):
+        """Zero-padded tensor-core packs of the layers on the 1/8 and 1/16 levels (built once per _ensure stamp); h16=True: the
+        hi-only packs of the fp16 route, cached beside the split ones."""
+        if getattr(self, "_tcp_stamp", None) != self._stamp:
+            self._tcp, self._tcp_stamp = {}, self._stamp
+        if h16 not in self._tcp:
+            self._tcp[h16] = self._build_tc_pack(h16)
+        return self._tcp[h16]
+
+    def _build_tc_pack(self, h16):
         P = self._pad32
 
         def vec(v, n, fill):
@@ -462,13 +480,14 @@ class StereoBaseAggregation(_Engine):
             w = layer._w5
             wp = w.new_zeros((P(w.shape[0]), P(w.shape[1])) + tuple(w.shape[2:]))
             wp[:w.shape[0], :w.shape[1]] = w
-            return (ops.pack_tc_weight(wp, 16, kw_order=kw_order), vec(layer.scale, wp.shape[0], 1.0), vec(layer.shift, wp.shape[0], 0.0))
+            return (ops.pack_tc_weight(wp, 16, kw_order=kw_order, h16=h16), vec(layer.scale, wp.shape[0], 1.0),
+                    vec(layer.shift, wp.shape[0], 0.0))
 
         def deconv(layer):
             w = layer._w5                                                   # (Cin, Cout, 4, 4, 4)
             wp = w.new_zeros((P(w.shape[0]), P(w.shape[1])) + tuple(w.shape[2:]))
             wp[:w.shape[0], :w.shape[1]] = w
-            return (ops.pack_tc_deconv_weight(wp), vec(layer.scale, wp.shape[1], 1.0), vec(layer.shift, wp.shape[1], 0.0))
+            return (ops.pack_tc_deconv_weight(wp, h16=h16), vec(layer.scale, wp.shape[1], 1.0), vec(layer.shift, wp.shape[1], 0.0))
 
         def cat1x1(layer):
             w = layer.w                                                     # (C0 + C1, Cout), both slabs Cout channels wide
@@ -505,13 +524,12 @@ class StereoBaseAggregation(_Engine):
                 sc, sh = vec(layer.scale, n, 1.0), vec(layer.shift, n, 0.0)
                 out = []
                 for lo, hi in bounds:
-                    wt = (ops.pack_tc_deconv_weight(wp[:, lo:hi].contiguous()) if transposed
-                          else ops.pack_tc_weight(wp[lo:hi].contiguous(), 16, kw_order=kw_order))
+                    wt = (ops.pack_tc_deconv_weight(wp[:, lo:hi].contiguous(), h16=h16) if transposed
+                          else ops.pack_tc_weight(wp[lo:hi].contiguous(), 16, kw_order=kw_order, h16=h16))
                     out.append((lo, wt, None if sc is None else sc[lo:hi].contiguous(), None if sh is None else sh[lo:hi].contiguous()))
                 return out
             t["conv3"] = (slices(l0, ((0, 96), (96, 160)), kw_order=(1, 0, 2)), slices(l1, ((0, 96), (96, 160))))
             t["conv3_up"] = slices(lu, ((0, 64), (64, 96)), transposed=True)
-        self._tcp, self._tcp_stamp = t, self._stamp
         return t
 
     def _level32_tc_ok(self, shape):
@@ -521,6 +539,16 @@ class StereoBaseAggregation(_Engine):
                     and ops.conv3d_tc_kc(160, 96, 16) == 16 and ops.conv3d_tc_kc(160, 64, 16) == 16
                     and ops.deconv3d_k4_tc_supported(160, 64, 16) and ops.deconv3d_k4_tc_supported(160, 32, 16))
 
+    def _h16_route_ok(self, shape):
+        """True when every layer of _call_tc has an fp16-activation kernel for an input volume of `shape` (the 1/32 level included)."""
+        b, c, d, h, w = shape
+        if not (self.tc_route_ok(shape) and self._level32_tc_ok(shape) and "conv3" in self._tc_pack()):
+            return False
+        pc, p2, p4 = self._pad32(c), self._pad32(2 * c), self._pad32(4 * c)
+        return (ops.conv3d_s2_tc_h16_supported(pc, p2, d, h, w) and ops.conv3d_tc_h16_supported(p2, p2, w // 2)
+                and ops.conv3d_s2_tc_h16_supported(p2, p4, d // 2, h // 2, w // 2) and ops.conv3d_tc_h16_supported(p4, p4, w // 4)
+                and ops.conv3d_s2_tc_h16_supported(p4, 96, d // 4, h // 4, w // 4) and ops.conv3d_tc_h16_supported(160, 96, w // 8))
+
     def _gate_nhwc(self, name, feat, channels):
         fa = self.att[name]                                                 # one launch: (B, H, W, C padded), padded channels 0
         if fa.a.w.shape[1] % 4 == 0 and fa.b.w.shape[1] % 4 == 0:
@@ -529,7 +557,9 @@ class StereoBaseAggregation(_Engine):
         return ops.to_ndhwc(fa(feat).unsqueeze(2), pad_to=channels).squeeze(1)
 
     def _call_tc(self, x, feats):
-        t = self._tc_pack()
+        """The tensor-core route; x fp32 (3xFP16 split kernels) or fp16 (H16 kernels: the ops dispatch on the activation dtype, every
+        intermediate stays fp16, the gates stay fp32)."""
+        t = self._tc_pack(x.dtype == torch.float16)
         c = x.shape[1]
         pc, p2, p4 = self._pad32(c), self._pad32(2 * c), self._pad32(4 * c)
         act = lambda name, i: self.conv[name][i][1]                         # noqa: E731
@@ -574,9 +604,12 @@ class StereoBaseAggregation(_Engine):
         return ops.deconv3d_k4_tc(conv1, wu, scu, shu, None, self.up["conv1_up"][1], out_ndhwc=False, cout_real=c)
 
     def __call__(self, x, features):
-        x = self._check(x)
+        h16 = self.precision == "fp16" and x.dtype == torch.float16
+        x = self._check(x, torch.float16 if h16 else torch.float32)
         self._ensure(x.device)
         feats = [self._check(f) for f in features]
+        if h16 and not self._h16_route_ok(x.shape):
+            x = x.float()
         if self.tc_route_ok(x.shape):
             mon = self._watch(x.device)
             out = self._call_tc(x, feats)

@@ -17,6 +17,8 @@
 // and StereoBase's sigmoid channel gate, so no elementwise pass ever touches HBM.
 #include <algorithm>
 
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 
 namespace osb {
@@ -658,11 +660,13 @@ static bool aligned16(const void* q) { return q == nullptr || (reinterpret_cast<
 // loads of both slabs.  Thread (warp w, lane l) owns voxels l, l+32, l+64, l+96 and the output channels [w, w+1) * COUT/4: per
 // four input channels it issues 4 LDS.128 of activations and COUT/4 broadcast LDS.128 of weights for 4 * COUT FMAs (FMA-bound, not
 // LSU-bound: the first version -- one voxel per thread, weights through L1 -- ran at 2.4 TFLOP/s).  Outputs leave through the tile.
-template <int CIN, int COUT>
+// H16: fp16 slabs in and fp16 out (StereoBase's fp16 hourglass route), fp32 weights and arithmetic; outputs are stored with
+// cvt.rn.satfinite and a magnitude beyond 65504 bumps the tensor-core overflow counter `overflow`.
+template <int CIN, int COUT, bool H16 = false>
 __global__ void __launch_bounds__(128) conv1x1_ndhwc_cat_kernel(const float* __restrict__ x0, const float* __restrict__ x1, int C0,
                                                                const float* __restrict__ w, const float* __restrict__ scale,
                                                                const float* __restrict__ shift, float* __restrict__ y, size_t V,
-                                                               int act) {
+                                                               int act, unsigned int* overflow) {
   constexpr int TS = CIN + 4;                       // tile row stride (floats): LDS.128 of a quarter warp hit distinct bank groups
   constexpr int F4 = CIN / 4, O4 = COUT / 4;
   constexpr int NC = COUT / 4;                      // output channels per warp
@@ -688,7 +692,15 @@ __global__ void __launch_bounds__(128) conv1x1_ndhwc_cat_kernel(const float* __r
     for (int f = threadIdx.x; f < 128 * F4; f += 128) {
       const int vox = f / F4, ch = f % F4;
       float4 t = make_float4(0.f, 0.f, 0.f, 0.f);
-      if (vox < nv)
+      if constexpr (H16) {
+        if (vox < nv) {
+          const __half* h0 = reinterpret_cast<const __half*>(x0), *h1 = reinterpret_cast<const __half*>(x1);
+          const uint2 u = ch < c0f4 ? __ldg(reinterpret_cast<const uint2*>(h0 + (v0 + vox) * C0) + ch)
+                                    : __ldg(reinterpret_cast<const uint2*>(h1 + (v0 + vox) * C1) + (ch - c0f4));
+          const float2 a = __half22float2(*reinterpret_cast<const __half2*>(&u.x)), b = __half22float2(*reinterpret_cast<const __half2*>(&u.y));
+          t = make_float4(a.x, a.y, b.x, b.y);
+        }
+      } else if (vox < nv)
         t = ch < c0f4 ? __ldg(reinterpret_cast<const float4*>(x0 + (v0 + vox) * C0) + ch)
                       : __ldg(reinterpret_cast<const float4*>(x1 + (v0 + vox) * C1) + (ch - c0f4));
       *reinterpret_cast<float4*>(tl + vox * TS + 4 * ch) = t;
@@ -736,20 +748,39 @@ __global__ void __launch_bounds__(128) conv1x1_ndhwc_cat_kernel(const float* __r
         *reinterpret_cast<float4*>(tl + (lane + 32 * v) * TS + cbase + 4 * q) = o;
       }
     __syncthreads();
-    float4* dst = reinterpret_cast<float4*>(y + v0 * COUT);
-    for (int f = threadIdx.x; f < 128 * O4; f += 128) {
-      const int vox = f / O4, ch = f % O4;
-      if (vox < nv) dst[f] = *reinterpret_cast<const float4*>(tl + vox * TS + 4 * ch);
+    if constexpr (H16) {
+      uint2* dst = reinterpret_cast<uint2*>(reinterpret_cast<__half*>(y) + v0 * COUT);
+      float amax = 0.f;
+      for (int f = threadIdx.x; f < 128 * O4; f += 128) {
+        const int vox = f / O4, ch = f % O4;
+        if (vox < nv) {
+          const float4 o = *reinterpret_cast<const float4*>(tl + vox * TS + 4 * ch);
+          amax = fmaxf(amax, fmaxf(fmaxf(fabsf(o.x), fabsf(o.y)), fmaxf(fabsf(o.z), fabsf(o.w))));
+          uint32_t lo, hi;
+          asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(lo) : "f"(o.y), "f"(o.x));
+          asm("cvt.rn.satfinite.f16x2.f32 %0, %1, %2;" : "=r"(hi) : "f"(o.w), "f"(o.z));
+          dst[f] = make_uint2(lo, hi);
+        }
+      }
+      if (amax > 65504.f) atomicAdd(overflow, 1u);
+    } else {
+      float4* dst = reinterpret_cast<float4*>(y + v0 * COUT);
+      for (int f = threadIdx.x; f < 128 * O4; f += 128) {
+        const int vox = f / O4, ch = f % O4;
+        if (vox < nv) dst[f] = *reinterpret_cast<const float4*>(tl + vox * TS + 4 * ch);
+      }
     }
   }
 }
 
-template <int CIN, int COUT>
+unsigned int* tc_overflow_flag();      // api.cu: sticky fp16-range counter of the tensor-core route (tc_common.cuh)
+
+template <int CIN, int COUT, bool H16 = false>
 static int launch_conv1x1_cat(const float* x0, const float* x1, int C0, const float* w, const float* scale, const float* shift, float* y,
-                              long long voxels, int act, cudaStream_t s) {
+                              long long voxels, int act, cudaStream_t s, unsigned int* overflow = nullptr) {
   constexpr size_t smem = ((size_t)CIN * COUT + (size_t)128 * (CIN + 4)) * sizeof(float);
   static_assert(smem <= 232448, "shared memory budget of one CTA exceeded");
-  auto kernel = conv1x1_ndhwc_cat_kernel<CIN, COUT>;
+  auto kernel = conv1x1_ndhwc_cat_kernel<CIN, COUT, H16>;
   static PerDeviceFlag configured;
   if (!configured.here()) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
@@ -762,7 +793,7 @@ static int launch_conv1x1_cat(const float* x0, const float* x1, int C0, const fl
   const long long tiles = (voxels + 127) / 128;
   const int per_sm = smem <= 113 * 1024 ? 2 : 1;
   const unsigned blocks = (unsigned)std::min<long long>(tiles, (long long)sm_count() * per_sm);
-  kernel<<<blocks, 128, smem, s>>>(x0, x1, C0, w, scale, shift, y, (size_t)voxels, act);
+  kernel<<<blocks, 128, smem, s>>>(x0, x1, C0, w, scale, shift, y, (size_t)voxels, act, overflow);
   count_launch();
   return check_launch("conv1x1_ndhwc_cat_kernel");
 }
@@ -847,6 +878,28 @@ int osb_conv1x1_ndhwc_cat_fwd(const float* x0, const float* x1, int C0, int C1, 
   if (Cin == 192 && Cout == 96) return launch_conv1x1_cat<192, 96>(x0, x1, C0, w_packed, scale, shift, y, voxels, act, s);
   if (Cin == 128 && Cout == 64) return launch_conv1x1_cat<128, 64>(x0, x1, C0, w_packed, scale, shift, y, voxels, act, s);
   set_error("conv1x1_ndhwc_cat: unsupported channels %d + %d -> %d (192 -> 96 and 128 -> 64 are instantiated)", C0, C1, Cout);
+  return OSB_EUNSUPPORTED;
+}
+
+int osb_conv1x1_ndhwc_cat_h16_fwd(const void* x0, const void* x1, int C0, int C1, const float* w_packed, const float* scale,
+                                  const float* shift, float* y, long long voxels, int Cout, int act, osb_stream_t stream) {
+  using namespace osb;
+  OSB_REQUIRE(x0 && x1 && w_packed && y, "conv1x1_ndhwc_cat_h16: null pointer");
+  OSB_REQUIRE(voxels > 0 && C0 > 0 && C1 > 0 && C0 % 4 == 0 && C1 % 4 == 0, "conv1x1_ndhwc_cat_h16: bad shape");
+  OSB_REQUIRE(act >= 0 && act <= 2, "conv1x1_ndhwc_cat_h16: unknown activation %d", act);
+  OSB_REQUIRE((reinterpret_cast<uintptr_t>(x0) & 7) == 0 && (reinterpret_cast<uintptr_t>(x1) & 7) == 0 &&
+                  (reinterpret_cast<uintptr_t>(y) & 7) == 0 && aligned16(w_packed),
+              "conv1x1_ndhwc_cat_h16: x0 / x1 / y must be 8-byte, w 16-byte aligned");
+  unsigned int* flag = tc_overflow_flag();
+  OSB_REQUIRE(flag, "conv1x1_ndhwc_cat_h16: cannot allocate the overflow flag");
+  cudaStream_t s = (cudaStream_t)stream;
+  const int Cin = C0 + C1;
+  const float* a = static_cast<const float*>(x0);
+  const float* b = static_cast<const float*>(x1);
+  float* o = y;
+  if (Cin == 192 && Cout == 96) return launch_conv1x1_cat<192, 96, true>(a, b, C0, w_packed, scale, shift, o, voxels, act, s, flag);
+  if (Cin == 128 && Cout == 64) return launch_conv1x1_cat<128, 64, true>(a, b, C0, w_packed, scale, shift, o, voxels, act, s, flag);
+  set_error("conv1x1_ndhwc_cat_h16: unsupported channels %d + %d -> %d (192 -> 96 and 128 -> 64 are instantiated)", C0, C1, Cout);
   return OSB_EUNSUPPORTED;
 }
 

@@ -498,9 +498,10 @@ __global__ void __launch_bounds__(TC_THREADS, 1) conv3d_tc_kernel(const TcParams
 
 // ---------------------------------------------------------------------------------------- layout conversion kernels
 // NCDHW -> NDHWC through a 32x32 shared-memory transpose (both sides coalesced).
-__global__ void __launch_bounds__(256) ncdhw_to_ndhwc_kernel(const float* __restrict__ x, float* __restrict__ y, int C, int Cp,
+template <typename T = float>       // float, or __half for the fp16 route (osb_ncdhw_to_ndhwc_pad_h16)
+__global__ void __launch_bounds__(256) ncdhw_to_ndhwc_kernel(const T* __restrict__ x, T* __restrict__ y, int C, int Cp,
                                                              size_t vol) {
-  __shared__ float tile[32][33];
+  __shared__ T tile[32][33];
   const int b = blockIdx.z;
   const size_t v0 = (size_t)blockIdx.x * 32;
   const int c0 = blockIdx.y * 32;
@@ -508,7 +509,7 @@ __global__ void __launch_bounds__(256) ncdhw_to_ndhwc_kernel(const float* __rest
   for (int i = ty; i < 32; i += 8) {
     const int c = c0 + i;
     const size_t v = v0 + tx;
-    tile[i][tx] = (c < C && v < vol) ? __ldg(x + ((size_t)b * C + c) * vol + v) : 0.f;
+    tile[i][tx] = (c < C && v < vol) ? __ldg(x + ((size_t)b * C + c) * vol + v) : T(0.f);
   }
   __syncthreads();
   for (int i = ty; i < 32; i += 8) {
@@ -545,6 +546,9 @@ int launch_tcg_dispatch(const float* x, const void* w, const float* scale, const
                         const float* gate = nullptr, int ystride = 0);
 int launch_tcg_dilated2(const float* x, const void* w, const float* scale, const float* shift, const float* residual, float* y,
                         int B, int Cin, int Cout, int H, int W, int act, int out_ndhwc, int res_ndhwc, cudaStream_t stream);
+bool tcg_h16_shape(int Cin, int Cout, int W);
+int launch_tcg_h16(const void* x, const void* w, const float* scale, const float* shift, const float* gate, float* y, int B, int Cin,
+                   int Cout, int D, int H, int W, int act, int ystride, cudaStream_t stream);
 
 }  // namespace osb
 
@@ -579,6 +583,17 @@ int osb_ncdhw_to_ndhwc_pad(const float* x, float* y, int B, int C, int Cpad, int
   ncdhw_to_ndhwc_kernel<<<grid, 256, 0, (cudaStream_t)stream>>>(x, y, C, Cpad, vol);
   count_launch();
   return check_launch("ncdhw_to_ndhwc_kernel");
+}
+
+int osb_ncdhw_to_ndhwc_pad_h16(const void* x, float* y, int B, int C, int Cpad, int D, int H, int W, osb_stream_t stream) {
+  using namespace osb;
+  OSB_REQUIRE(x && y, "ncdhw_to_ndhwc_h16: null pointer");
+  OSB_REQUIRE(B > 0 && C > 0 && Cpad >= C && D > 0 && H > 0 && W > 0 && B <= 65535, "ncdhw_to_ndhwc_h16: bad shape");
+  const size_t vol = (size_t)D * H * W;
+  dim3 grid((unsigned)((vol + 31) / 32), (Cpad + 31) / 32, B);
+  ncdhw_to_ndhwc_kernel<__half><<<grid, 256, 0, (cudaStream_t)stream>>>(static_cast<const __half*>(x), reinterpret_cast<__half*>(y), C, Cpad, vol);
+  count_launch();
+  return check_launch("ncdhw_to_ndhwc_kernel<half>");
 }
 
 int osb_ncdhw_to_ndhwc(const float* x, float* y, int B, int C, int D, int H, int W, osb_stream_t stream) {
@@ -645,6 +660,39 @@ int osb_conv3d_k3_tc_cs_fwd(const float* x_ndhwc, const void* w_split, const flo
                             const float* gate_nhwc, float* y, int B, int Cin, int Cout, int D, int H, int W, int act, int ystride,
                             osb_stream_t stream) {
   return conv3d_k3_tc_impl(x_ndhwc, w_split, scale, shift, residual, y, B, Cin, Cout, D, H, W, act, 1, 1, 0, stream, gate_nhwc, ystride);
+}
+
+// ---- fp16 activations (H16 instantiations of conv3d_tcg.cu): channels-last fp16 x and y, fp32 gate, no residual
+static int conv3d_k3_tc_h16_impl(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, const float* gate,
+                                 float* y, int B, int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
+  using namespace osb;
+  OSB_REQUIRE(x_ndhwc && w_split && y, "conv3d_k3_tc_h16: null pointer");
+  OSB_REQUIRE(B > 0 && D > 0 && H > 0, "conv3d_k3_tc_h16: empty shape");
+  OSB_REQUIRE(tcg_h16_shape(Cin, Cout, W), "conv3d_k3_tc_h16: unsupported shape Cin=%d Cout=%d W=%d", Cin, Cout, W);
+  OSB_REQUIRE(act >= 0 && act <= 2, "conv3d_k3_tc_h16: unknown activation %d", act);
+  OSB_REQUIRE(ystride == 0 || (W == 16 && ystride >= Cout && ystride % 4 == 0), "conv3d_k3_tc_h16: bad channel stride %d", ystride);
+  OSB_REQUIRE((reinterpret_cast<uintptr_t>(x_ndhwc) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_split) & 15) == 0 &&
+                  (reinterpret_cast<uintptr_t>(y) & 7) == 0 && (reinterpret_cast<uintptr_t>(gate) & 15) == 0,
+              "conv3d_k3_tc_h16: x, w and gate must be 16-byte, y 8-byte aligned");
+  return launch_tcg_h16(x_ndhwc, w_split, scale, shift, gate, y, B, Cin, Cout, D, H, W, act, ystride, (cudaStream_t)stream);
+}
+
+int osb_conv3d_tc_h16_supported(int Cin, int Cout, int W) { return osb::tcg_h16_shape(Cin, Cout, W) ? 1 : 0; }
+
+int osb_conv3d_k3_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                             int Cout, int D, int H, int W, int act, osb_stream_t stream) {
+  return conv3d_k3_tc_h16_impl(x_ndhwc, w_split, scale, shift, nullptr, y, B, Cin, Cout, D, H, W, act, 0, stream);
+}
+
+int osb_conv3d_k3_tc_gate_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, const float* gate_nhwc,
+                                  float* y, int B, int Cin, int Cout, int D, int H, int W, int act, osb_stream_t stream) {
+  OSB_REQUIRE(gate_nhwc, "conv3d_k3_tc_gate_h16: null gate");
+  return conv3d_k3_tc_h16_impl(x_ndhwc, w_split, scale, shift, gate_nhwc, y, B, Cin, Cout, D, H, W, act, 0, stream);
+}
+
+int osb_conv3d_k3_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, const float* gate_nhwc,
+                                float* y, int B, int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
+  return conv3d_k3_tc_h16_impl(x_ndhwc, w_split, scale, shift, gate_nhwc, y, B, Cin, Cout, D, H, W, act, ystride, stream);
 }
 
 int osb_conv3d_k3_tc_ncdhw_fwd(const float* x_ncdhw, const void* w_split, const float* scale, const float* shift,

@@ -23,12 +23,12 @@
 namespace osb {
 
 struct TcdcParams {
-  const float* x;          // (B, D, H, W, Cin) channels-last
+  const float* x;          // (B, D, H, W, Cin) channels-last (fp16 in the H16 instantiations)
   const void* w;           // fp16 [3 kd][Cin/KC][3 kh][3*Cout][KC hi | KC lo]  (ops.pack_tc_weight)
   const float* scale;
   const float* shift;
   const float* residual;
-  float* y;
+  float* y;                // fp16 in the H16 instantiations
   int B, D, H, Cin;        // INPUT extent D x H x W; output is 2D x 2H x 2W
   int act;
   float kappa;       // expected round-towards-zero loss per accumulating MMA (tc_common.cuh)
@@ -111,9 +111,11 @@ __device__ __forceinline__ ItemDc decode_dc(const TcdcParams& p, int it) {
   return w;
 }
 
-template <int COUT, int KC, int W, int TILES, bool GW = false, int KS = 3>
+// H16: fp16 activations in and out, one hi x hi MMA per k-step (see conv3d_tcg.cu)
+template <int COUT, int KC, int W, int TILES, bool GW = false, int KS = 3, bool H16 = false>
 __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 1) conv3d_tcdc_kernel(const TcdcParams p) {
   using C = TcdcCfg<COUT, KC, W, TILES, GW, KS>;
+  using A = TcAct<H16>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint8_t* a_buf = smem + C::A_OFF;
@@ -204,9 +206,13 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
                   const uint64_t db0 = dbase | (uint64_t)(b16 + (bslot * C::B_SLICE) / 16);
 #pragma unroll
                   for (int ks = 0; ks < C::KSTEPS; ++ks) {
-                    mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
-                    mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
-                    mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                    if constexpr (H16) {
+                      mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);
+                    } else {
+                      mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
+                      mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
+                      mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                    }
                   }
                 }
                 __syncwarp();
@@ -243,24 +249,28 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
     float amax = 0.f;
     uint32_t ubase = 0;                              // global index of the current phase's first unit
     int first = lw;                                  // this warp's first local unit index in the current phase: (ubase + first) % NLW == lw
-    auto fill = [&](const float* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
+    auto fill = [&](const typename A::T* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
       // base: this lane's address for load 0; load j covers operand rows VPL*j .. VPL*j + VPL - 1 = columns (VPL*j) % W ..
       // of tile row (VPL*j) / W, read from image row h_first + h_step * tile row (rstride / cstride floats per tile row / column).
       // General widths: col0 = INPUT column of load 0 (columns >= Wp are zero: beyond the image).
-      float4 v[NLD];
+      typename A::V v[NLD];
 #pragma unroll
       for (int j = 0; j < NLD; ++j) {
         const int hin = h_first + h_step * ((VPL * j) / W);
         const size_t off = (size_t)((VPL * j) / W) * rstride + (size_t)((VPL * j) % W) * cstride;
         bool ok = hin >= 0 && hin < p.H;
         if (GW) ok = ok && (unsigned)(col0 + VPL * j) < (unsigned)Wp;
-        v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        if constexpr (H16) v[j] = ok ? __ldg(reinterpret_cast<const uint2*>(base + (ptrdiff_t)off)) : make_uint2(0u, 0u);
+        else v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
       const uint32_t slot = u % C::STAGES, ph = (u / C::STAGES) & 1;   // u = global unit index
       mbar_wait_relaxed(&a_empty[slot], ph ^ 1);
       uint8_t* tile = a_buf + slot * C::UNIT_BYTES;
 #pragma unroll
-      for (int j = 0; j < NLD; ++j) stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      for (int j = 0; j < NLD; ++j) {
+        if constexpr (H16) stage_f16_hi<KC>(tile, v0 + VPL * j, c, v[j]);
+        else stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      }
       fence_proxy_async();
       mbar_arrive(&a_ready[slot]);
     };
@@ -269,7 +279,7 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
       for (int kd = 0; kd < KS; ++kd) {
         if (!kd_valid(w.od, kd, p.D)) continue;
         const int id = (w.od + 1 - kd) >> 1;         // input plane feeding output plane od through tap kd
-        const float* plane = p.x + ((size_t)w.b * p.D + id) * p.H * (size_t)Wp * p.Cin;
+        const typename A::T* plane = reinterpret_cast<const typename A::T*>(p.x) + ((size_t)w.b * p.D + id) * p.H * (size_t)Wp * p.Cin;
         const int col0 = w.ct * C::CSTEP + v0;       // INPUT column of this lane's first load (whole-row kernels: v0)
         // valid kh taps of this row parity in issue order: k3: ph 0 -> {1}, ph 1 -> {0, 2};  k4: ph 0 -> {1, 3}, ph 1 -> {0, 2}
         const int nkh = (KS == 4 || w.ph) ? 2 : 1, kh0 = w.ph ? 0 : 1;
@@ -281,7 +291,7 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
             // operand row v = input voxel (row j0 + t*R + v / W + (ph + 1 - kh) / 2, column v % W): output row 2j + ph gathers
             // tap kh from input row j + (ph + 1 - kh) / 2  (k3: +1 for kh = 0; k4: +1 for kh = 0, -1 for kh = 3)
             const int h_first = w.j0 + t * C::R + ((w.ph + 1 - kh) >> 1);
-            const float* base = plane + ((ptrdiff_t)h_first * Wp + col0) * p.Cin + ch * KC + c * 4;
+            const typename A::T* base = plane + ((ptrdiff_t)h_first * Wp + col0) * p.Cin + ch * KC + c * 4;
             fill(base, (size_t)Wp * p.Cin, (size_t)p.Cin, h_first, 1, ubase + j, col0);
           }
           ubase += upp;
@@ -301,11 +311,12 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
     const int Do = 2 * p.D, Ho = 2 * p.H;
     const int Wo = 2 * Wp;
     uint32_t itc = 0, exc = 0;
+    float yamax = 0.f;                               // H16: largest stored magnitude (fp16 saturation at 65504)
     for (int it = blockIdx.x; it < p.items; it += gridDim.x, ++itc) {
       const ItemDc w = decode_dc<C>(p, it);
       const int ntiles = min(TILES, (p.H - w.j0 + C::R - 1) / C::R);
       // tap pairs of this parity class: (1 or 2 kd) x (1 or 2 kh); each adds chunks x k-steps x 3 MMAs (tc_common.cuh: rz_kappa)
-      const float corr = 1.f + p.kappa * (float)(w.nkd * (KS == 4 ? 2 : w.ph + 1) * nchunk * C::KSTEPS * 3);
+      const float corr = 1.f + p.kappa * (float)(w.nkd * (KS == 4 ? 2 : w.ph + 1) * nchunk * C::KSTEPS * A::TERMS);
       // general widths: input column of this thread's tile column; the halo column and columns beyond the image are not stored
       const int col = GW ? w.ct * C::CSTEP + m : wcol;
       const bool cvalid = !GW || (m < C::CSTEP && col < Wp);
@@ -421,7 +432,13 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
           }
           // coalesced channels-last path (BN/residual/act inside); W < 32: the warp's two input rows map to output rows that are
           // not adjacent in memory -> per-thread stores below
-          if (W >= 32 && live && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {
+          if (H16 && W >= 32 && live && p.out_ndhwc) {    // fp16 output, no residual (checked at the entry point)
+            __half* y0 = reinterpret_cast<__half*>(p.y) + (vox - 2 * lane) * YS + cg;
+            store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, ev, y0, nullptr, 2 * YS, s_scale + cg, s_shift + cg, p.act, vmask,
+                                nullptr, &yamax);
+            store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, od_, y0 + YS, nullptr, 2 * YS, s_scale + cg, s_shift + cg, p.act, vmask,
+                                nullptr, &yamax);
+          } else if (!H16 && W >= 32 && live && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {
             // lane k owns output voxels (vox0 + 2k) and (vox0 + 2k + 1): two transposes with a 2-voxel lane stride
             float* y0 = p.y + (vox - 2 * lane) * YS + cg;
             const float* r0 = p.residual ? p.residual + (vox - 2 * lane) * YS + cg : nullptr;
@@ -463,7 +480,27 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
                 od_[i] = od_[i] > 0.f ? od_[i] : 0.01f * od_[i];
               }
             }
-            if (p.out_ndhwc) {
+            if constexpr (H16) {
+              __half* yh = reinterpret_cast<__half*>(p.y);
+              if (p.out_ndhwc) {
+                uint2* yp = reinterpret_cast<uint2*>(yh + vox * YS + cg);
+                uint2* yq = reinterpret_cast<uint2*>(yh + (vox + 1) * YS + cg);
+#pragma unroll
+                for (int i = 0; i < 32; ++i) yamax = fmaxf(yamax, fmaxf(fabsf(ev[i]), fabsf(od_[i])));
+#pragma unroll
+                for (int i = 0; i < 8; ++i) {
+                  yp[i] = make_uint2(cvt_f16x2_sat(ev[4 * i], ev[4 * i + 1]), cvt_f16x2_sat(ev[4 * i + 2], ev[4 * i + 3]));
+                  yq[i] = make_uint2(cvt_f16x2_sat(od_[4 * i], od_[4 * i + 1]), cvt_f16x2_sat(od_[4 * i + 2], od_[4 * i + 3]));
+                }
+              } else {
+#pragma unroll
+                for (int i = 0; i < 32; ++i)           // columns 2w, 2w+1 as one fp16 pair
+                  if (cg + i < p.cout_real) {
+                    yamax = fmaxf(yamax, fmaxf(fabsf(ev[i]), fabsf(od_[i])));
+                    *reinterpret_cast<uint32_t*>(yh + ncdhw0 + (size_t)(cg + i) * plane) = cvt_f16x2_sat(ev[i], od_[i]);
+                  }
+              }
+            } else if (p.out_ndhwc) {
               float4* yp = reinterpret_cast<float4*>(p.y + vox * YS + cg);
               float4* yq = reinterpret_cast<float4*>(p.y + (vox + 1) * YS + cg);
 #pragma unroll
@@ -484,6 +521,7 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
         mbar_arrive(&acc_empty[t]);
       }
     }
+    if constexpr (H16) tc_report_overflow(p.overflow, yamax);
   }
   // ---------------------------------------------------------------------------------------------- weight-slice producer
   // One elected lane streams the pre-swizzled (kd, chunk, kh) slices with 1-D TMA bulk copies into the two buffers of tap kh, up
@@ -517,10 +555,10 @@ __global__ void __launch_bounds__(TcdcCfg<COUT, KC, W, TILES, GW, KS>::THREADS, 
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
-template <int COUT, int KC, int W, int TILES, bool GW = false, int KS = 3>
+template <int COUT, int KC, int W, int TILES, bool GW = false, int KS = 3, bool H16 = false>
 static int launch_tcdc(TcdcParams& p, cudaStream_t stream) {
   using C = TcdcCfg<COUT, KC, W, TILES, GW, KS>;
-  auto kernel = conv3d_tcdc_kernel<COUT, KC, W, TILES, GW, KS>;
+  auto kernel = conv3d_tcdc_kernel<COUT, KC, W, TILES, GW, KS, H16>;
   static PerDeviceFlag configured;
   if (!configured.here()) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
@@ -615,6 +653,45 @@ static int deconv3d_k4_tc_impl(const float* x_ndhwc, const void* w_split, const 
   if (W == 16 && Cout == 32) return launch_tcdc<32, 16, 16, 4, false, 4>(p, s);
   if (W == 32) return launch_tcdc<64, 16, 32, 2, false, 4>(p, s);
   return launch_tcdc<32, 16, 64, 4, false, 4>(p, s);
+}
+
+// ---- fp16 activations (H16 instantiations of the k4 kernel): same shapes as osb_deconv3d_k4_tc_supported, no residual
+static int deconv3d_k4_tc_h16_impl(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                   int Cin, int Cout, int cout_real, int D, int H, int W, int act, int out_ndhwc, int ystride,
+                                   osb_stream_t stream) {
+  using namespace osb;
+  OSB_REQUIRE(x_ndhwc && w_split && y, "deconv3d_k4_tc_h16: null pointer");
+  OSB_REQUIRE(B > 0 && D > 0 && H > 0, "deconv3d_k4_tc_h16: empty shape");
+  OSB_REQUIRE(osb_deconv3d_k4_tc_supported(Cin, Cout, W), "deconv3d_k4_tc_h16: unsupported shape Cin=%d Cout=%d W=%d", Cin, Cout, W);
+  OSB_REQUIRE(act >= 0 && act <= 2, "deconv3d_k4_tc_h16: unknown activation %d", act);
+  OSB_REQUIRE(ystride == 0 || (W == 16 && ystride >= Cout && ystride % 4 == 0 && out_ndhwc), "deconv3d_k4_tc_h16: bad channel stride %d",
+              ystride);
+  OSB_REQUIRE(cout_real >= 1 && cout_real <= Cout && (out_ndhwc == 0 || cout_real == Cout),
+              "deconv3d_k4_tc_h16: only NCDHW outputs may hold fewer (%d) channels than the packed %d", cout_real, Cout);
+  OSB_REQUIRE((reinterpret_cast<uintptr_t>(x_ndhwc) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_split) & 15) == 0 &&
+                  (reinterpret_cast<uintptr_t>(y) & 7) == 0,
+              "deconv3d_k4_tc_h16: x and w must be 16-byte, y 8-byte aligned");
+  TcdcParams p{};
+  p.cout_real = cout_real, p.ystride = ystride;
+  p.x = static_cast<const float*>(x_ndhwc), p.w = w_split, p.scale = scale, p.shift = shift, p.y = y;
+  p.B = B, p.D = D, p.H = H, p.Cin = Cin, p.act = act, p.out_ndhwc = out_ndhwc ? 1 : 0, p.res_ndhwc = 1;
+  p.kappa = rz_kappa(), p.overflow = tc_overflow_flag();
+  OSB_REQUIRE(p.overflow, "tensor-core conv: cannot allocate the overflow flag");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (W == 16 && Cout == 64) return launch_tcdc<64, 16, 16, 2, false, 4, true>(p, s);
+  if (W == 16 && Cout == 32) return launch_tcdc<32, 16, 16, 4, false, 4, true>(p, s);
+  if (W == 32) return launch_tcdc<64, 16, 32, 2, false, 4, true>(p, s);
+  return launch_tcdc<32, 16, 64, 4, false, 4, true>(p, s);
+}
+
+int osb_deconv3d_k4_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                               int Cout, int cout_real, int D, int H, int W, int act, int out_ndhwc, osb_stream_t stream) {
+  return deconv3d_k4_tc_h16_impl(x_ndhwc, w_split, scale, shift, y, B, Cin, Cout, cout_real, D, H, W, act, out_ndhwc, 0, stream);
+}
+
+int osb_deconv3d_k4_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                  int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
+  return deconv3d_k4_tc_h16_impl(x_ndhwc, w_split, scale, shift, y, B, Cin, Cout, Cout, D, H, W, act, 1, ystride, stream);
 }
 
 int osb_deconv3d_k3_tc_fwd(const float* x_ndhwc, const void* w_split, const float* scale, const float* shift,

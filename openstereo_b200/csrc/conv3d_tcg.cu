@@ -20,13 +20,13 @@
 namespace osb {
 
 struct TcgParams {
-  const float* x;          // (B, D, H, W, Cin) channels-last
+  const float* x;          // (B, D, H, W, Cin) channels-last (fp16 in the H16 instantiations)
   const void* w;           // fp16 [3 kd][Cin/KC][3 kh][3*Cout][KC hi | KC lo]  (ops.pack_tc_weight)
   const float* scale;
   const float* shift;
   const float* residual;
   const float* gate;       // optional (B, H, W, Cout) channels-last multiplier applied after the activation (FeatureAtt), NDHWC output only
-  float* y;
+  float* y;                // fp16 in the H16 instantiations (channels-last only)
   int B, D, H, Cin;
   int act;
   float kappa;       // expected round-towards-zero loss per accumulating MMA (tc_common.cuh)
@@ -100,9 +100,12 @@ struct TcgCfg {
   }
 };
 
-template <int COUT, int KC, int W, int TILES, int DIL = 1, bool GW = false, bool GATE = false>
+// H16: fp16 activations in and out, one hi x hi MMA per k-step (tc_common.cuh: TcAct); the shared-memory layout is the split
+// kernel's, the lo halves of the operand rows are left unused.
+template <int COUT, int KC, int W, int TILES, int DIL = 1, bool GW = false, bool GATE = false, bool H16 = false>
 __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 1) conv3d_tcg_kernel(const TcgParams p) {
   using C = TcgCfg<COUT, KC, W, TILES, DIL, GW>;
+  using A = TcAct<H16>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint8_t* a_buf = smem + C::A_OFF;
@@ -201,9 +204,13 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
                     const uint64_t db0 = dbase | (uint64_t)(b16 + (((phc & 1) * 3 + kh) * C::B_SLICE + mm * C::NPER * C::ROWB) / 16);
 #pragma unroll
                     for (int ks = 0; ks < C::KSTEPS; ++ks) {
-                      mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
-                      mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
-                      mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                      if constexpr (H16) {
+                        mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);
+                      } else {
+                        mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
+                        mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
+                        mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                      }
                     }
                   }
                 }
@@ -241,24 +248,28 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
     float amax = 0.f;
     uint32_t ubase = 0;                              // global index of the current phase's first unit
     int first = lw;                                  // this warp's first local unit index in the current phase: (ubase + first) % NLW == lw
-    auto fill = [&](const float* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
+    auto fill = [&](const typename A::T* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
       // base: this lane's address for load 0; load j covers operand rows VPL*j .. VPL*j + VPL - 1 = columns (VPL*j) % W ..
       // of tile row (VPL*j) / W, read from image row h_first + h_step * tile row (rstride / cstride floats per tile row / column).
       // General widths: col0 = image column of load 0 (may be -HALO .. or beyond Wr: those columns are zero padding).
-      float4 v[NLD];
+      typename A::V v[NLD];
 #pragma unroll
       for (int j = 0; j < NLD; ++j) {
         const int hin = h_first + h_step * ((VPL * j) / W);
         const size_t off = (size_t)((VPL * j) / W) * rstride + (size_t)((VPL * j) % W) * cstride;
         bool ok = hin >= 0 && hin < p.H;
         if (GW) ok = ok && (unsigned)(col0 + VPL * j) < (unsigned)Wp;
-        v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        if constexpr (H16) v[j] = ok ? __ldg(reinterpret_cast<const uint2*>(base + (ptrdiff_t)off)) : make_uint2(0u, 0u);
+        else v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
       const uint32_t slot = u % C::STAGES, ph = (u / C::STAGES) & 1;   // u = global unit index
       mbar_wait_relaxed(&a_empty[slot], ph ^ 1);
       uint8_t* tile = a_buf + slot * C::UNIT_BYTES;
 #pragma unroll
-      for (int j = 0; j < NLD; ++j) stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      for (int j = 0; j < NLD; ++j) {
+        if constexpr (H16) stage_f16_hi<KC>(tile, v0 + VPL * j, c, v[j]);
+        else stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      }
       fence_proxy_async();
       mbar_arrive(&a_ready[slot]);
     };
@@ -272,13 +283,13 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
       for (int kd = 0; kd < 3; ++kd) {
         const int din = d + kd - 1;
         if (din < 0 || din >= p.D) continue;
-        const float* plane = p.x + ((size_t)b * p.D + din) * p.H * (size_t)Wp * p.Cin;
+        const typename A::T* plane = reinterpret_cast<const typename A::T*>(p.x) + ((size_t)b * p.D + din) * p.H * (size_t)Wp * p.Cin;
         for (int ch = 0; ch < nchunk; ++ch) {
 #pragma unroll 1
           for (int j = first; j < C::NU; j += C::NLW) {
             // unit = R consecutive image rows starting at h0 + s: operand row v is voxel (h0 + s) * W + v of the plane
             const int s = C::unit_s(j);
-            const float* base = plane + ((ptrdiff_t)(h0 + s) * Wp + col0) * p.Cin + ch * KC + c * 4;
+            const typename A::T* base = plane + ((ptrdiff_t)(h0 + s) * Wp + col0) * p.Cin + ch * KC + c * 4;
             fill(base, (size_t)Wp * p.Cin, (size_t)p.Cin, h0 + s, 1, ubase + j, col0);
           }
           ubase += C::NU;
@@ -296,6 +307,7 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
     const bool has_left_q = ((q * 32) % W) != 0;     // the quadrant to the left continues the same image row
     const bool has_right_q = (((q + 1) * 32) % W) != 0;
     uint32_t itc = 0, exc = 0;
+    float yamax = 0.f;                               // H16: largest stored magnitude (fp16 saturation at 65504)
     for (int it = blockIdx.x; it < p.items; it += gridDim.x, ++itc) {
       const int ct = it % ctiles;
       const int hb = (it / ctiles) % p.hblocks;
@@ -307,7 +319,7 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
       const int col = GW ? ct * C::CSTEP - C::HALO + m : wcol;
       const bool cvalid = !GW || (m >= C::HALO && m < 128 - C::HALO && col < Wp);
       const uint32_t vmask = GW ? __ballot_sync(0xffffffffu, cvalid) : 0xffffffffu;
-      const float corr = 1.f + p.kappa * (float)(((d > 0) + 1 + (d + 1 < p.D)) * nchunk * 3 * C::KSTEPS * 3);   // tc_common.cuh: rz_kappa
+      const float corr = 1.f + p.kappa * (float)(((d > 0) + 1 + (d + 1 < p.D)) * nchunk * 3 * C::KSTEPS * A::TERMS);   // tc_common.cuh: rz_kappa
       for (int t = 0; t < ntiles; ++t) {
         const int h = h0 + t * C::R + rr;
         const bool live = h < p.H;
@@ -371,12 +383,16 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
           }
           // voxels of this warp that exist (W < 32: the warp spans two image rows, the second may lie below the image)
           const uint32_t vm = (W < 32) ? __ballot_sync(0xffffffffu, live) : (live ? vmask : 0u);
-          if (vm && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {     // coalesced channels-last path (BN/residual/act inside)
+          if (H16 && vm) {                             // channels-last fp16 output, no residual (checked at the entry point)
+            const ptrdiff_t gvox = GATE ? ((ptrdiff_t)b * p.H + h) * Wp + col - lane : 0;
+            store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, out, reinterpret_cast<__half*>(p.y) + (vox - lane) * YS + cg, nullptr, YS,
+                                s_scale + cg, s_shift + cg, p.act, vm, (GATE && p.gate) ? p.gate + gvox * YS + cg : nullptr, &yamax);
+          } else if (!H16 && vm && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {     // coalesced channels-last path (BN/residual/act inside)
             const ptrdiff_t gvox = GATE ? ((ptrdiff_t)b * p.H + h) * Wp + col - lane : 0;   // (B, H, W) index of lane 0's voxel
             store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, out, p.y + (vox - lane) * YS + cg,
                                 p.residual ? p.residual + (vox - lane) * YS + cg : nullptr, YS, s_scale + cg, s_shift + cg, p.act,
                                 vm, (GATE && p.gate) ? p.gate + gvox * YS + cg : nullptr);
-          } else if (live && cvalid) {
+          } else if (!H16 && live && cvalid) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) out[i] = fmaf(out[i], s_scale[cg + i], s_shift[cg + i]);
             if (p.residual) {
@@ -415,6 +431,7 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
         mbar_arrive(&acc_empty[t]);
       }
     }
+    if constexpr (H16) tc_report_overflow(p.overflow, yamax);
   }
   // ---------------------------------------------------------------------------------------------- weight-slice producer
   // One elected lane streams the pre-swizzled (kd, chunk, kh) slices with 1-D TMA bulk copies into the two buffer sets, up to a
@@ -447,10 +464,10 @@ __global__ void __launch_bounds__(TcgCfg<COUT, KC, W, TILES, DIL, GW>::THREADS, 
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
-template <int COUT, int KC, int W, int TILES, int DIL = 1, bool GW = false, bool GATE = false>
+template <int COUT, int KC, int W, int TILES, int DIL = 1, bool GW = false, bool GATE = false, bool H16 = false>
 static int launch_tcg(TcgParams& p, cudaStream_t stream) {
   using C = TcgCfg<COUT, KC, W, TILES, DIL, GW>;
-  auto kernel = conv3d_tcg_kernel<COUT, KC, W, TILES, DIL, GW, GATE>;
+  auto kernel = conv3d_tcg_kernel<COUT, KC, W, TILES, DIL, GW, GATE, H16>;
   if (!GATE && p.gate) {
     set_error("conv3d_tcg: no gated instantiation for Cout=%d W=%d", COUT, W);
     return OSB_EUNSUPPORTED;
@@ -517,6 +534,26 @@ int launch_tcg_dispatch(const float* x, const void* w, const float* scale, const
   if (Cout == 64) return launch_tcg<64, 16, 128, 2, 1, true>(p, stream);
   if (Cout == 128) return launch_tcg<128, 16, 128, 1, 1, true>(p, stream);
   return -1;
+}
+
+// fp16 activations (H16 instantiations): the whole-row shapes of StereoBase's hourglass at W' = 128 -- 1/8 level (W = 64, Cout = 64),
+// 1/16 level (W = 32, Cout = 96), 1/32 level channel slices (W = 16, Cout = 96 | 64); channels-last in and out, no residual.
+bool tcg_h16_shape(int Cin, int Cout, int W) {
+  return Cin % 16 == 0 && Cin >= 16 && ((W == 64 && Cout == 64) || (W == 32 && Cout == 96) || (W == 16 && (Cout == 96 || Cout == 64)));
+}
+
+int launch_tcg_h16(const void* x, const void* w, const float* scale, const float* shift, const float* gate, float* y, int B, int Cin,
+                   int Cout, int D, int H, int W, int act, int ystride, cudaStream_t stream) {
+  TcgParams p{};
+  p.x = static_cast<const float*>(x), p.w = w, p.scale = scale, p.shift = shift, p.gate = gate, p.y = y;
+  p.ystride = ystride;
+  p.B = B, p.D = D, p.H = H, p.Cin = Cin, p.act = act, p.out_ndhwc = 1, p.res_ndhwc = 1;
+  p.kappa = rz_kappa(), p.overflow = tc_overflow_flag();
+  if (!p.overflow) return OSB_ECUDA;
+  if (W == 64) return gate ? launch_tcg<64, 16, 64, 2, 1, false, true, true>(p, stream) : launch_tcg<64, 16, 64, 2, 1, false, false, true>(p, stream);
+  if (W == 32) return gate ? launch_tcg<96, 16, 32, 1, 1, false, true, true>(p, stream) : launch_tcg<96, 16, 32, 1, 1, false, false, true>(p, stream);
+  if (Cout == 96) return launch_tcg<96, 16, 16, 1, 1, false, true, true>(p, stream);
+  return launch_tcg<64, 16, 16, 2, 1, false, true, true>(p, stream);
 }
 
 // dilated (2) one-plane variant for the 2D backbone: same parameters with D == 1

@@ -17,12 +17,12 @@
 namespace osb {
 
 struct Tcs2Params {
-  const float* x;          // (B, D, H, W, Cin) channels-last
+  const float* x;          // (B, D, H, W, Cin) channels-last (fp16 in the H16 instantiations)
   const void* w;           // fp16 [3 kd][Cin/KC][3 kh][3*Cout][KC hi | KC lo]  (ops.pack_tc_weight)
   const float* scale;
   const float* shift;
   const float* residual;
-  float* y;
+  float* y;                // fp16 in the H16 instantiations (channels-last only)
   int B, D, H, Cin;        // INPUT extent D x H x (2*WO); output is D/2 x H/2 x WO
   int act;
   float kappa;       // expected round-towards-zero loss per accumulating MMA (tc_common.cuh)
@@ -67,9 +67,11 @@ struct Tcs2Cfg {
   static_assert(COUT % 16 == 0 && 2 * COUT <= 256, "invalid UMMA N");
 };
 
-template <int COUT, int KC, int W, int TILES, bool GW = false>
+// H16: fp16 activations in and out, one hi x hi MMA per k-step (see conv3d_tcg.cu)
+template <int COUT, int KC, int W, int TILES, bool GW = false, bool H16 = false>
 __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) conv3d_tcs2_kernel(const Tcs2Params p) {
   using C = Tcs2Cfg<COUT, KC, W, TILES, GW>;
+  using A = TcAct<H16>;
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
   uint8_t* a_buf = smem + C::A_OFF;
@@ -165,9 +167,13 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
                     const uint32_t idesc = par ? idesc_o : idesc_e;
 #pragma unroll
                     for (int ks = 0; ks < C::KSTEPS; ++ks) {
-                      mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
-                      mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
-                      mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                      if constexpr (H16) {
+                        mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);
+                      } else {
+                        mma_f16(acc, da0 + C::LO + 2 * ks, db0 + 2 * ks, idesc, ks > 0 ? 1u : accum);   // small terms first
+                        mma_f16(acc, da0 + 2 * ks, db0 + C::LO + 2 * ks, idesc, 1);
+                        mma_f16(acc, da0 + 2 * ks, db0 + 2 * ks, idesc, 1);
+                      }
                     }
                   }
                   __syncwarp();
@@ -206,24 +212,28 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
     const int Do = p.D / 2;
     uint32_t ubase = 0;                              // global index of the current phase's first unit
     int first = lw;                                  // this warp's first local unit index in the current phase: (ubase + first) % NLW == lw
-    auto fill = [&](const float* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
+    auto fill = [&](const typename A::T* base, size_t rstride, size_t cstride, int h_first, int h_step, uint32_t u, int col0) {
       // base: this lane's address for load 0; load j covers operand rows VPL*j .. VPL*j + VPL - 1 = columns (VPL*j) % W ..
       // of tile row (VPL*j) / W, read from image row h_first + h_step * tile row (rstride / cstride floats per tile row / column).
       // General widths: col0 = OUTPUT column of load 0 (-1 = the left halo; columns outside [0, Wp) are zero padding).
-      float4 v[NLD];
+      typename A::V v[NLD];
 #pragma unroll
       for (int j = 0; j < NLD; ++j) {
         const int hin = h_first + h_step * ((VPL * j) / W);
         const size_t off = (size_t)((VPL * j) / W) * rstride + (size_t)((VPL * j) % W) * cstride;
         bool ok = hin >= 0 && hin < p.H;
         if (GW) ok = ok && (unsigned)(col0 + VPL * j) < (unsigned)Wp;
-        v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
+        if constexpr (H16) v[j] = ok ? __ldg(reinterpret_cast<const uint2*>(base + (ptrdiff_t)off)) : make_uint2(0u, 0u);
+        else v[j] = ok ? __ldg(reinterpret_cast<const float4*>(base + (ptrdiff_t)off)) : make_float4(0.f, 0.f, 0.f, 0.f);
       }
       const uint32_t slot = u % C::STAGES, ph = (u / C::STAGES) & 1;   // u = global unit index
       mbar_wait_relaxed(&a_empty[slot], ph ^ 1);
       uint8_t* tile = a_buf + slot * C::UNIT_BYTES;
 #pragma unroll
-      for (int j = 0; j < NLD; ++j) stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      for (int j = 0; j < NLD; ++j) {
+        if constexpr (H16) stage_f16_hi<KC>(tile, v0 + VPL * j, c, v[j]);
+        else stage_f16_split<KC>(tile, v0 + VPL * j, c, v[j], amax);
+      }
       fence_proxy_async();
       mbar_arrive(&a_ready[slot]);
     };
@@ -237,14 +247,14 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
       for (int kd = 0; kd < 3; ++kd) {
         const int din = 2 * od + kd - 1;
         if (din < 0 || din >= p.D) continue;
-        const float* plane = p.x + ((size_t)b * p.D + din) * p.H * (size_t)WI * p.Cin;
+        const typename A::T* plane = reinterpret_cast<const typename A::T*>(p.x) + ((size_t)b * p.D + din) * p.H * (size_t)WI * p.Cin;
         for (int ch = 0; ch < nchunk; ++ch) {
 #pragma unroll 1
           for (int j = first; j < C::NU; j += C::NLW) {       // local unit index = (t * 3 + kh) * 2 + par
             const int t = j / 6, kh = (j >> 1) % 3, par = j & 1;
             // operand row v = output voxel (row h0 + t*R + v / W, column v % W) reading input (2*row + kh - 1, 2*col + par)
             const int h_first = 2 * (h0 + t * C::R) + kh - 1;
-            const float* base = plane + ((ptrdiff_t)h_first * WI + 2 * col0 + par) * p.Cin + ch * KC + c * 4;
+            const typename A::T* base = plane + ((ptrdiff_t)h_first * WI + 2 * col0 + par) * p.Cin + ch * KC + c * 4;
             fill(base, (size_t)2 * WI * p.Cin, (size_t)2 * p.Cin, h_first, 2, ubase + j, col0);
           }
           ubase += C::NU;
@@ -262,6 +272,7 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
     const bool has_left_q = ((q * 32) % W) != 0;     // the quadrant to the left continues the same image row
     const int Do = p.D / 2, Ho = p.H / 2;
     uint32_t itc = 0, exc = 0;
+    float yamax = 0.f;                               // H16: largest stored magnitude (fp16 saturation at 65504)
     for (int it = blockIdx.x; it < p.items; it += gridDim.x, ++itc) {
       const int ct = it % ctiles;
       const int hb = (it / ctiles) % p.hblocks;
@@ -274,7 +285,7 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
       const bool cvalid = !GW || (m >= C::HALO && col < Wp);
       const uint32_t vmask = GW ? __ballot_sync(0xffffffffu, cvalid) : 0xffffffffu;
       // input planes 2d-1, 2d, 2d+1: the first is missing for d = 0 (tc_common.cuh: rz_kappa)
-      const float corr = 1.f + p.kappa * (float)(((d > 0) + 1 + (2 * d + 1 < p.D)) * nchunk * 3 * C::KSTEPS * 3);
+      const float corr = 1.f + p.kappa * (float)(((d > 0) + 1 + (2 * d + 1 < p.D)) * nchunk * 3 * C::KSTEPS * A::TERMS);
       for (int t = 0; t < ntiles; ++t) {
         mbar_wait_relaxed(&acc_full[t], itc & 1);
         tc_fence_after();
@@ -320,11 +331,14 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
             }
           }
           const uint32_t vm = (W < 32) ? __ballot_sync(0xffffffffu, live) : (live ? vmask : 0u);   // voxels of this warp that exist
-          if (vm && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {     // coalesced channels-last path (BN/residual/act inside)
+          if (H16 && vm) {                             // channels-last fp16 output, no residual (checked at the entry point)
+            store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, out, reinterpret_cast<__half*>(p.y) + (vox - lane) * YS + cg, nullptr, YS,
+                                s_scale + cg, s_shift + cg, p.act, vm, nullptr, &yamax);
+          } else if (!H16 && vm && p.out_ndhwc && (!p.residual || p.res_ndhwc)) {     // coalesced channels-last path (BN/residual/act inside)
             store_ndhwc_chunk32(tpose + q * TP_WARP_FLOATS, lane, out, p.y + (vox - lane) * YS + cg,
                                 p.residual ? p.residual + (vox - lane) * YS + cg : nullptr, YS, s_scale + cg, s_shift + cg, p.act,
                                 vm);
-          } else if (live && cvalid) {
+          } else if (!H16 && live && cvalid) {
 #pragma unroll
             for (int i = 0; i < 32; ++i) out[i] = fmaf(out[i], s_scale[cg + i], s_shift[cg + i]);
             if (p.residual) {
@@ -363,6 +377,7 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
         mbar_arrive(&acc_empty[t]);
       }
     }
+    if constexpr (H16) tc_report_overflow(p.overflow, yamax);
   }
   // ---------------------------------------------------------------------------------------------- weight-slice producer
   // One elected lane streams the pre-swizzled (kd, chunk, kh) slices with 1-D TMA bulk copies into the two buffer sets, up to a
@@ -395,10 +410,10 @@ __global__ void __launch_bounds__(Tcs2Cfg<COUT, KC, W, TILES, GW>::THREADS, 1) c
   if (warp == 0) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem), "r"(512));
 }
 
-template <int COUT, int KC, int W, int TILES, bool GW = false>
+template <int COUT, int KC, int W, int TILES, bool GW = false, bool H16 = false>
 static int launch_tcs2(Tcs2Params& p, cudaStream_t stream) {
   using C = Tcs2Cfg<COUT, KC, W, TILES, GW>;
-  auto kernel = conv3d_tcs2_kernel<COUT, KC, W, TILES, GW>;
+  auto kernel = conv3d_tcs2_kernel<COUT, KC, W, TILES, GW, H16>;
   static PerDeviceFlag configured;
   if (!configured.here()) {
     cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)C::SMEM);
@@ -483,5 +498,48 @@ int osb_conv3d_k3_s2_tc_fwd(const float* x_ndhwc, const void* w_split, const flo
 int osb_conv3d_k3_s2_tc_cs_fwd(const float* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
                                int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
   return conv3d_k3_s2_tc_impl(x_ndhwc, w_split, scale, shift, nullptr, y, B, Cin, Cout, D, H, W, act, 1, 1, ystride, stream);
+}
+
+// ---- fp16 activations (H16 instantiations): the whole-row shapes of StereoBase's hourglass, channels-last, no residual
+static bool s2_h16_shape(int Cin, int Cout, int W) {
+  return Cin % 16 == 0 && Cin >= 16 && ((W == 128 && Cout == 64) || (W == 64 && Cout == 96) || (W == 32 && (Cout == 96 || Cout == 64)));
+}
+
+static int conv3d_k3_s2_tc_h16_impl(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                    int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
+  using namespace osb;
+  OSB_REQUIRE(x_ndhwc && w_split && y, "conv3d_k3_s2_tc_h16: null pointer");
+  OSB_REQUIRE(B > 0 && D > 0 && H > 0 && D % 2 == 0 && H % 2 == 0, "conv3d_k3_s2_tc_h16: bad shape");
+  OSB_REQUIRE(s2_h16_shape(Cin, Cout, W), "conv3d_k3_s2_tc_h16: unsupported shape Cin=%d Cout=%d W=%d", Cin, Cout, W);
+  OSB_REQUIRE(act >= 0 && act <= 2, "conv3d_k3_s2_tc_h16: unknown activation %d", act);
+  OSB_REQUIRE(ystride == 0 || (W == 32 && ystride >= Cout && ystride % 4 == 0), "conv3d_k3_s2_tc_h16: bad channel stride %d", ystride);
+  OSB_REQUIRE((reinterpret_cast<uintptr_t>(x_ndhwc) & 15) == 0 && (reinterpret_cast<uintptr_t>(w_split) & 15) == 0 &&
+                  (reinterpret_cast<uintptr_t>(y) & 7) == 0,
+              "conv3d_k3_s2_tc_h16: x and w must be 16-byte, y 8-byte aligned");
+  Tcs2Params p{};
+  p.x = static_cast<const float*>(x_ndhwc), p.w = w_split, p.scale = scale, p.shift = shift, p.y = y;
+  p.B = B, p.D = D, p.H = H, p.Cin = Cin, p.act = act, p.out_ndhwc = 1, p.res_ndhwc = 1;
+  p.kappa = rz_kappa(), p.overflow = tc_overflow_flag();
+  p.ystride = ystride;
+  OSB_REQUIRE(p.overflow, "tensor-core conv: cannot allocate the overflow flag");
+  cudaStream_t s = (cudaStream_t)stream;
+  if (W == 32 && Cout == 96) return launch_tcs2<96, 16, 16, 1, false, true>(p, s);
+  if (W == 32) return launch_tcs2<64, 16, 16, 2, false, true>(p, s);
+  if (W == 128) return launch_tcs2<64, 16, 64, 2, false, true>(p, s);
+  return launch_tcs2<96, 16, 32, 1, false, true>(p, s);
+}
+
+int osb_conv3d_s2_tc_h16_supported(int Cin, int Cout, int D, int H, int W) {
+  return (D % 2 == 0 && H % 2 == 0 && s2_h16_shape(Cin, Cout, W)) ? 1 : 0;
+}
+
+int osb_conv3d_k3_s2_tc_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B, int Cin,
+                                int Cout, int D, int H, int W, int act, osb_stream_t stream) {
+  return conv3d_k3_s2_tc_h16_impl(x_ndhwc, w_split, scale, shift, y, B, Cin, Cout, D, H, W, act, 0, stream);
+}
+
+int osb_conv3d_k3_s2_tc_cs_h16_fwd(const void* x_ndhwc, const void* w_split, const float* scale, const float* shift, float* y, int B,
+                                   int Cin, int Cout, int D, int H, int W, int act, int ystride, osb_stream_t stream) {
+  return conv3d_k3_s2_tc_h16_impl(x_ndhwc, w_split, scale, shift, y, B, Cin, Cout, D, H, W, act, ystride, stream);
 }
 }

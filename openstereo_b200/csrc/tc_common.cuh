@@ -1,6 +1,8 @@
 // Shared device helpers of the tcgen05 convolution kernels (conv3d_tc.cu: W = 128 specialisation; conv3d_tcg.cu: generic
 // multi-row tiles).  See conv3d_tc.cu for the design notes.
 #pragma once
+#include <cuda_fp16.h>
+
 #include "common.cuh"
 
 namespace osb {
@@ -175,6 +177,27 @@ __device__ __forceinline__ void stage_f16_split(uint8_t* tile, int row, int q, c
   *reinterpret_cast<uint2*>(tile + swz_offset<KC>(row, q >> 1) + sub) = hi;
   *reinterpret_cast<uint2*>(tile + swz_offset<KC>(row, KC / 8 + (q >> 1)) + sub) = lo;
 }
+// 16-bit activation route (H16 instantiations, DESIGN.md section 4.11): the activations already ARE fp16 (the caller ran the model
+// under autocast and asked for 16-bit arithmetic), so four channels arrive as 8 bytes and go to the hi half of the row unchanged --
+// no TC_ACT_SCALE, no split, the lo half of the row is never read (one MMA per k-step, A hi x B hi).
+template <int KC>
+__device__ __forceinline__ void stage_f16_hi(uint8_t* tile, int row, int q, const uint2 v) {
+  *reinterpret_cast<uint2*>(tile + swz_offset<KC>(row, q >> 1) + ((q & 1) << 3)) = v;
+}
+// activation element / 4-channel load type of the loaders and products per k-step of the two routes
+template <bool H16>
+struct TcAct {
+  using T = float;
+  using V = float4;
+  static constexpr int TERMS = 3;      // lo*hi + hi*lo + hi*hi
+};
+template <>
+struct TcAct<true> {
+  using T = __half;
+  using V = uint2;
+  static constexpr int TERMS = 1;      // hi*hi
+};
+
 // Lane -> operand row inside a warp-wide load of VPL = 128 / KC voxels (KC/4 lanes each), permuted so that the two STS.64 of
 // stage_f16_split are bank-conflict free per half-warp: SWIZZLE_128B rows (KC = 32) must differ in bit 2, SWIZZLE_64B rows
 // (KC = 16) must be {r, r+1, r+4, r+5}.  Global loads stay whole 16-byte chunks of whole voxels either way.
@@ -207,9 +230,13 @@ constexpr int TP_BYTES = 4 * TP_WARP_FLOATS * 4;    // four epilogue warps
 // the last tile beyond the image; whole-row tiles pass all ones and the tests fold away).
 // gate0: optional channels-last multiplier of lane 0's voxel (same voxel stride), applied AFTER the activation -- FeatureAtt's
 // sigmoid(att) * cv of stereobase/hourglass.py:80-99 / igev_blocks.py:35-48 with the gate stored as (B, H, W, C).
-__device__ __forceinline__ void store_ndhwc_chunk32(float* tbuf, int lane, const float (&sum)[32], float* y0, const float* res0,
+// T = __half (H16 instantiations): the fp32 results are stored with cvt.rn.satfinite; *amax tracks their largest magnitude so the
+// caller can count values that saturated at +-65504 (tc_report_overflow).
+template <typename T = float>
+__device__ __forceinline__ void store_ndhwc_chunk32(float* tbuf, int lane, const float (&sum)[32], T* y0, const float* res0,
                                                     size_t vstride, const float* sc, const float* sh, int act,
-                                                    uint32_t vmask = 0xffffffffu, const float* gate0 = nullptr) {
+                                                    uint32_t vmask = 0xffffffffu, const float* gate0 = nullptr,
+                                                    float* amax = nullptr) {
   const int c4 = 4 * (lane & 7), sub = lane >> 3;
   __syncwarp();                                     // the previous chunk's readers are done with the tile
   float4* row = reinterpret_cast<float4*>(tbuf + lane * TP_STRIDE);
@@ -251,9 +278,19 @@ __device__ __forceinline__ void store_ndhwc_chunk32(float* tbuf, int lane, const
       o[j].x *= g.x, o[j].y *= g.y, o[j].z *= g.z, o[j].w *= g.w;
     }
   }
+  if constexpr (sizeof(T) == 2) {
 #pragma unroll
-  for (int j = 0; j < 8; ++j)
-    if ((vmask >> (4 * j + sub)) & 1u) *reinterpret_cast<float4*>(y0 + (size_t)(4 * j + sub) * vstride + c4) = o[j];
+    for (int j = 0; j < 8; ++j)
+      if ((vmask >> (4 * j + sub)) & 1u) {
+        *amax = fmaxf(*amax, fmaxf(fmaxf(fabsf(o[j].x), fabsf(o[j].y)), fmaxf(fabsf(o[j].z), fabsf(o[j].w))));
+        *reinterpret_cast<uint2*>(y0 + (size_t)(4 * j + sub) * vstride + c4) =
+            make_uint2(cvt_f16x2_sat(o[j].x, o[j].y), cvt_f16x2_sat(o[j].z, o[j].w));
+      }
+  } else {
+#pragma unroll
+    for (int j = 0; j < 8; ++j)
+      if ((vmask >> (4 * j + sub)) & 1u) *reinterpret_cast<float4*>(y0 + (size_t)(4 * j + sub) * vstride + c4) = o[j];
+  }
 }
 
 }  // namespace osb

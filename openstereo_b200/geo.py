@@ -33,7 +33,8 @@ class CombinedGeoEncodingVolume:
         """All-pairs row correlation (gru_blocks.py:222-229): a batched fp32 GEMM, left to cuBLAS."""
         b, _, h, w1 = fmap1.shape
         w2 = fmap2.shape[-1]
-        corr = torch.einsum('aijk,aijh->ajkh', fmap1, fmap2)
+        with torch.autocast("cuda", enabled=False):                 # fp32 also when the model is evaluated under autocast
+            corr = torch.einsum('aijk,aijh->ajkh', fmap1, fmap2)
         return corr.reshape(b, h, w1, 1, w2).contiguous()
 
 

@@ -480,13 +480,15 @@ def f16_split(w):
 class TcWeight:
     """A conv weight packed for the tcgen05 kernels: `data` fp16 [3 kd][Cin/kc][3 kh][3*Cout (kw-major)][kc hi | kc lo] of
     w * 2^e_c with the 16-byte chunks of every row stored in UMMA swizzle order (pack_tc_weight), and `inv` = 2^-(e_c + TC_ACT_SCALE_LOG2) per output channel -- the exact factor the epilogue must apply.
-    `cout` is the packed row count per kw slice (narrow heads are zero-padded to 16), `cout_real` the layer's channels."""
-    __slots__ = ("data", "inv", "kc", "cout", "cout_real", "ksize", "_eff")
+    `cout` is the packed row count per kw slice (narrow heads are zero-padded to 16), `cout_real` the layer's channels.
+    `h16`: a hi-only pack for the fp16-activation kernels (pack_tc_weight(..., h16=True)): lo halves zero, `inv` = 2^-e_c."""
+    __slots__ = ("data", "inv", "kc", "cout", "cout_real", "ksize", "h16", "_eff")
 
-    def __init__(self, data, inv, kc, cout, cout_real=None, ksize=3):
+    def __init__(self, data, inv, kc, cout, cout_real=None, ksize=3, h16=False):
         self.data, self.inv, self.kc, self.cout, self._eff = data, inv, kc, cout, None
         self.cout_real = cout if cout_real is None else cout_real
         self.ksize = ksize                                                  # 3, or 4 for the k4-s2 transposed conv
+        self.h16 = bool(h16)
 
     def eff_scale(self, scale):
         """Epilogue scale vector: folded-BN scale (or 1) times the exact power-of-two un-scaling of this weight."""
@@ -499,10 +501,12 @@ class TcWeight:
         return self._eff[1]
 
 
-def pack_tc_weight(weight, kc=None, kw_order=(0, 1, 2), pad_cout_to=None):
+def pack_tc_weight(weight, kc=None, kw_order=(0, 1, 2), pad_cout_to=None, h16=False):
     """(Cout, Cin, k, k, k) fp32 Conv3d parameter (k = 3, or 4 for the k4-s2 transposed conv) -> TcWeight (see there).  Per output
     channel the weights are scaled by the power of two that puts max |w| into [2^14, 2^15) (exact; undone by TcWeight.inv), then
-    split with f16_split.  kw_order lists the kw slices in the order the kernel stacks them along N."""
+    split with f16_split.  kw_order lists the kw slices in the order the kernel stacks them along N.
+    h16=True: the pack of the fp16-activation kernels -- hi = rn_fp16(w * 2^e) only (lo halves zero: one MMA per product), same
+    power-of-two scaling (no weight becomes subnormal), inv = 2^-e (the activations are not scaled)."""
     w = weight.detach().float()
     cout_real, cin = w.shape[:2]
     k = int(w.shape[2])
@@ -515,7 +519,11 @@ def pack_tc_weight(weight, kc=None, kw_order=(0, 1, 2), pad_cout_to=None):
     _, ex = torch.frexp(amax)                                           # amax = m * 2^ex, m in [0.5, 1)
     e = torch.where(amax > 0, TC_WEIGHT_TOP_LOG2 - ex, torch.zeros_like(ex)).clamp(-40, 40)
     ws = torch.ldexp(w, e.view(-1, 1, 1, 1, 1))
-    hi, lo = f16_split(ws)
+    if h16:
+        hi = ws.contiguous().to(torch.float16)
+        lo = torch.zeros_like(hi)
+    else:
+        hi, lo = f16_split(ws)
     both = torch.stack((hi, lo), 0)                                    # (2, co, ci, kd, kh, kw)
     both = both[..., list(kw_order)]                                   # stride-2 kernel wants kw slices as (1, 0, 2)
     both = both.contiguous().view(2, cout, cin // kc, kc, k, k, k)     # (half, co, chunk, ci, kd, kh, kw)
@@ -531,8 +539,20 @@ def pack_tc_weight(weight, kc=None, kw_order=(0, 1, 2), pad_cout_to=None):
     data = data.view(k, cin // kc, k, k * cout, cpr, 8)
     data = torch.gather(data, 4, src.view(1, 1, 1, k * cout, cpr, 1).expand(k, cin // kc, k, k * cout, cpr, 8).contiguous())
     data = data.reshape(k, cin // kc, k, k * cout, 2 * kc).contiguous()
-    inv = torch.ldexp(torch.ones_like(amax), -(e + TC_ACT_SCALE_LOG2))
-    return TcWeight(data, inv.contiguous(), kc, cout, cout_real, ksize=k)
+    inv = torch.ldexp(torch.ones_like(amax), -(e if h16 else e + TC_ACT_SCALE_LOG2))
+    return TcWeight(data, inv.contiguous(), kc, cout, cout_real, ksize=k, h16=h16)
+
+
+def _is_h16(x, w_split=None, what="x"):
+    """Activation dtype dispatch of the tensor-core ops: True for fp16 (the _h16 entry points, which need an h16 weight pack), False
+    for fp32; any other dtype, or a weight pack of the other kind, raises."""
+    if x.dtype not in (torch.float32, torch.float16):
+        raise TypeError("%s: the tensor-core ops take float32 or float16 activations, got %s" % (what, x.dtype))
+    h16 = x.dtype == torch.float16
+    if w_split is not None and bool(getattr(w_split, "h16", False)) != h16:
+        raise ValueError("%s is %s but the weight pack is %s: pack with pack_tc_weight(..., h16=%s)"
+                         % (what, x.dtype, "hi-only (h16=True)" if w_split.h16 else "hi/lo split (h16=False)", h16))
+    return h16
 
 
 def _tc_args(w_split, cin, kc, scale):
@@ -544,14 +564,17 @@ def _tc_args(w_split, cin, kc, scale):
 
 
 def to_ndhwc(x, pad_to=None):
-    """(B,C,D,H,W) -> (B,D,H,W,C) contiguous fp32, on the device; pad_to > C appends zero channels (channel plans that are not
-    multiples of 16 run on the tensor-core kernels zero-padded)."""
-    assert x.is_cuda and x.dtype == torch.float32 and x.is_contiguous() and x.dim() == 5
+    """(B,C,D,H,W) -> (B,D,H,W,C) contiguous, same dtype (fp32 or fp16), on the device; pad_to > C appends zero channels (channel
+    plans that are not multiples of 16 run on the tensor-core kernels zero-padded)."""
+    assert x.is_cuda and x.is_contiguous() and x.dim() == 5
+    h16 = _is_h16(x)
     b, c, d, h, w = x.shape
     cp = c if pad_to is None else int(pad_to)
     assert cp >= c
-    y = torch.empty((b, d, h, w, cp), dtype=torch.float32, device=x.device)
-    if cp == c:
+    y = torch.empty((b, d, h, w, cp), dtype=x.dtype, device=x.device)
+    if h16:
+        _call("osb_ncdhw_to_ndhwc_pad_h16", x.data_ptr(), y.data_ptr(), b, c, cp, d, h, w, _stream(y))
+    elif cp == c:
         _call("osb_ncdhw_to_ndhwc", x.data_ptr(), y.data_ptr(), b, c, d, h, w, _stream(y))
     else:
         _call("osb_ncdhw_to_ndhwc_pad", x.data_ptr(), y.data_ptr(), b, c, cp, d, h, w, _stream(y))
@@ -561,8 +584,13 @@ def to_ndhwc(x, pad_to=None):
 def conv3d_k3_tc(x_ndhwc, w_split, scale=None, shift=None, residual=None, act=ACT_NONE, out_ndhwc=True, res_ndhwc=True,
                  in_ncdhw=False, gate=None):
     """3x3x3 stride-1 conv + folded BN + residual + activation on the tensor cores.  x_ndhwc: (B,D,H,W,Cin), or the NCDHW
-    tensor (B,Cin,D,H,W) with in_ncdhw=True (W = 128 layers only: the cost volume goes in as the volume kernel wrote it)."""
-    assert x_ndhwc.is_cuda and x_ndhwc.dtype == torch.float32 and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
+    tensor (B,Cin,D,H,W) with in_ncdhw=True (W = 128 layers only: the cost volume goes in as the volume kernel wrote it).
+    fp16 x (with an h16 weight pack): fp16 channels-last output, no residual, fp32 gate (osb_conv3d_k3_tc_h16_fwd)."""
+    assert x_ndhwc.is_cuda and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
+    if _is_h16(x_ndhwc, w_split):
+        if residual is not None or not out_ndhwc or in_ncdhw:
+            raise ValueError("conv3d_k3_tc: fp16 activations take channels-last in and out and no residual")
+        return _conv3d_k3_tc_h16(x_ndhwc, w_split, scale, shift, act, gate)
     if in_ncdhw:
         b, cin, d, h, w = x_ndhwc.shape
     else:
@@ -590,18 +618,50 @@ def conv3d_k3_tc(x_ndhwc, w_split, scale=None, shift=None, residual=None, act=AC
     return y
 
 
+def _conv3d_k3_tc_h16(x, w_split, scale, shift, act, gate):
+    b, d, h, w, cin = x.shape
+    cout = w_split.cout
+    if not conv3d_tc_h16_supported(cin, cout, w):
+        raise NotImplementedError("conv3d_k3_tc: no fp16 kernel for Cin=%d Cout=%d W=%d" % (cin, cout, w))
+    wptr, scale = _tc_args(w_split, cin, 16, scale)
+    y = torch.empty((b, d, h, w, cout), dtype=torch.float16, device=x.device)
+    if gate is not None:
+        assert tuple(gate.shape) == (b, h, w, cout) and gate.is_contiguous() and gate.dtype == torch.float32 and gate.is_cuda
+        _call("osb_conv3d_k3_tc_gate_h16_fwd", x.data_ptr(), wptr, _ptr(scale), _ptr(shift), gate.data_ptr(), y.data_ptr(), b, cin, cout,
+              d, h, w, act, _stream(y))
+    else:
+        _call("osb_conv3d_k3_tc_h16_fwd", x.data_ptr(), wptr, _ptr(scale), _ptr(shift), y.data_ptr(), b, cin, cout, d, h, w, act, _stream(y))
+    return y
+
+
+def conv3d_tc_h16_supported(cin, cout, w):
+    """True when a stride-1 fp16-activation kernel serves this shape (include/openstereo_b200.h: osb_conv3d_tc_h16_supported)."""
+    return bool(_lib.lib.osb_conv3d_tc_h16_supported(int(cin), int(cout), int(w)))
+
+
+def conv3d_s2_tc_h16_supported(cin, cout, d, h, w):
+    return bool(_lib.lib.osb_conv3d_s2_tc_h16_supported(int(cin), int(cout), int(d), int(h), int(w)))
+
+
 def conv3d_s2_tc_supported(cin, cout, d, h, w):
     return bool(_lib.lib.osb_conv3d_s2_tc_supported(int(cin), int(cout), int(d), int(h), int(w)))
 
 
 def conv3d_k3_s2_tc(x_ndhwc, w_split, scale=None, shift=None, residual=None, act=ACT_NONE, out_ndhwc=False, res_ndhwc=False):
     """3x3x3 STRIDE-2 conv + folded BN + residual + activation on the tensor cores.  x_ndhwc: (B,D,H,W,Cin), even D,H,W;
-    w_split = pack_tc_weight(weight, 16, kw_order=(1, 0, 2))."""
-    assert x_ndhwc.is_cuda and x_ndhwc.dtype == torch.float32 and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
+    w_split = pack_tc_weight(weight, 16, kw_order=(1, 0, 2)).  fp16 x (h16 pack): fp16 channels-last output, no residual."""
+    assert x_ndhwc.is_cuda and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
     b, d, h, w, cin = x_ndhwc.shape
     cout = w_split.cout
     wptr, scale = _tc_args(w_split, cin, 16, scale)
     do, ho, wo = d // 2, h // 2, w // 2
+    if _is_h16(x_ndhwc, w_split):
+        if residual is not None or not out_ndhwc:
+            raise ValueError("conv3d_k3_s2_tc: fp16 activations take channels-last in and out and no residual")
+        y = torch.empty((b, do, ho, wo, cout), dtype=torch.float16, device=x_ndhwc.device)
+        _call("osb_conv3d_k3_s2_tc_h16_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), y.data_ptr(), b, cin, cout, d, h, w, act,
+              _stream(y))
+        return y
     shape = (b, do, ho, wo, cout) if out_ndhwc else (b, cout, do, ho, wo)
     y = torch.empty(shape, dtype=torch.float32, device=x_ndhwc.device)
     if residual is not None:
@@ -616,13 +676,13 @@ def deconv3d_tc_supported(cin, cout, w):
     return bool(_lib.lib.osb_deconv3d_tc_supported(int(cin), int(cout), int(w)))
 
 
-def pack_tc_deconv_weight(weight):
+def pack_tc_deconv_weight(weight, h16=False):
     """(Cin, Cout, 3, 3, 3) ConvTranspose3d parameter -> TcWeight, 16-channel chunks, kw slices ordered (1, 2, 0):
     even output columns come from tap 1, odd ones from taps 2 (same input column) and 0 (next input column).
     (Cin, Cout, 4, 4, 4) (k4 s2 p1): kw slices (1, 3, 2, 0) -- even columns taps 1 (same input column) and 3 (previous one), odd
     columns taps 2 (same) and 0 (next)."""
     w = weight.detach().float().permute(1, 0, 2, 3, 4).contiguous()
-    return pack_tc_weight(w, 16, kw_order=(1, 2, 0) if w.shape[2] == 3 else (1, 3, 2, 0))
+    return pack_tc_weight(w, 16, kw_order=(1, 2, 0) if w.shape[2] == 3 else (1, 3, 2, 0), h16=h16)
 
 
 def deconv3d_k4_tc_supported(cin, cout, w):
@@ -632,13 +692,22 @@ def deconv3d_k4_tc_supported(cin, cout, w):
 def deconv3d_k4_tc(x_ndhwc, w_split, scale=None, shift=None, residual=None, act=ACT_NONE, out_ndhwc=True, res_ndhwc=True,
                    cout_real=None):
     """ConvTranspose3d(k4, s2, p1) + folded BN + residual + activation on the tensor cores.  x_ndhwc: (B,D,H,W,Cin); cout_real <
-    packed Cout (zero-padded channel plan) is allowed for an NCDHW output, which then holds only the real channels."""
-    assert x_ndhwc.is_cuda and x_ndhwc.dtype == torch.float32 and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
+    packed Cout (zero-padded channel plan) is allowed for an NCDHW output, which then holds only the real channels.
+    fp16 x (h16 pack): fp16 output, no residual."""
+    assert x_ndhwc.is_cuda and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
     b, d, h, w, cin = x_ndhwc.shape
     cout = w_split.cout
     creal = cout if cout_real is None else int(cout_real)
     assert w_split.ksize == 4 and (out_ndhwc is False or creal == cout)
     wptr, scale = _tc_args(w_split, cin, 16, scale)
+    if _is_h16(x_ndhwc, w_split):
+        if residual is not None:
+            raise ValueError("deconv3d_k4_tc: fp16 activations take no residual")
+        shape = (b, 2 * d, 2 * h, 2 * w, cout) if out_ndhwc else (b, creal, 2 * d, 2 * h, 2 * w)
+        y = torch.empty(shape, dtype=torch.float16, device=x_ndhwc.device)
+        _call("osb_deconv3d_k4_tc_h16_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), y.data_ptr(), b, cin, cout, creal, d, h, w,
+              act, 1 if out_ndhwc else 0, _stream(y))
+        return y
     shape = (b, 2 * d, 2 * h, 2 * w, cout) if out_ndhwc else (b, creal, 2 * d, 2 * h, 2 * w)
     y = torch.empty(shape, dtype=torch.float32, device=x_ndhwc.device)
     if residual is not None:
@@ -652,29 +721,38 @@ def deconv3d_k4_tc(x_ndhwc, w_split, scale=None, shift=None, residual=None, act=
 def tc_slice(kind, x_ndhwc, w_split, scale, shift, y, coff, act=ACT_NONE, gate=None):
     """One output-channel SLICE of a tensor-core conv (include/openstereo_b200.h: *_cs_fwd): channels [coff, coff + w_split.cout) of
     the preallocated channels-last `y` (..., Ctot).  kind: "s1" (3x3x3 stride 1, optional (B,H,W,Ctot) gate), "s2" (stride 2) or
-    "dc4" (ConvTranspose3d k4 s2 p1).  scale / shift: this slice's folded BN."""
-    assert x_ndhwc.is_cuda and x_ndhwc.dtype == torch.float32 and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
-    assert y.is_contiguous() and y.dtype == torch.float32 and y.dim() == 5
+    "dc4" (ConvTranspose3d k4 s2 p1).  scale / shift: this slice's folded BN.  fp16 x and y (h16 pack): the _cs_h16 entry points,
+    gate stays fp32."""
+    assert x_ndhwc.is_cuda and x_ndhwc.is_contiguous() and x_ndhwc.dim() == 5
+    assert y.is_contiguous() and y.dim() == 5
+    h16 = _is_h16(x_ndhwc, w_split)
+    if y.dtype != x_ndhwc.dtype:
+        raise ValueError("tc_slice: x is %s but y is %s" % (x_ndhwc.dtype, y.dtype))
     b, d, h, w, cin = x_ndhwc.shape
     cout, ctot = w_split.cout, y.shape[-1]
     assert 0 <= coff and coff + cout <= ctot and coff % 4 == 0
     wptr, scale = _tc_args(w_split, cin, 16, scale)
-    yp = y.data_ptr() + 4 * coff
+    yp = y.data_ptr() + y.element_size() * coff
+    sfx = "_h16_fwd" if h16 else "_fwd"
     if kind == "s1":
         assert tuple(y.shape[:4]) == (b, d, h, w)
         gp = None
         if gate is not None:
-            assert tuple(gate.shape) == (b, h, w, ctot) and gate.is_contiguous()
+            assert tuple(gate.shape) == (b, h, w, ctot) and gate.is_contiguous() and gate.dtype == torch.float32
             gp = gate.data_ptr() + 4 * coff
-        _call("osb_conv3d_k3_tc_cs_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), None, gp, yp, b, cin, cout, d, h, w, act,
-              ctot, _stream(y))
+        if h16:
+            _call("osb_conv3d_k3_tc_cs_h16_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), gp, yp, b, cin, cout, d, h, w, act,
+                  ctot, _stream(y))
+        else:
+            _call("osb_conv3d_k3_tc_cs_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), None, gp, yp, b, cin, cout, d, h, w, act,
+                  ctot, _stream(y))
     elif kind == "s2":
         assert tuple(y.shape[:4]) == (b, d // 2, h // 2, w // 2) and gate is None
-        _call("osb_conv3d_k3_s2_tc_cs_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), yp, b, cin, cout, d, h, w, act, ctot,
+        _call("osb_conv3d_k3_s2_tc_cs" + sfx, x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), yp, b, cin, cout, d, h, w, act, ctot,
               _stream(y))
     else:
         assert kind == "dc4" and tuple(y.shape[:4]) == (b, 2 * d, 2 * h, 2 * w) and gate is None and w_split.ksize == 4
-        _call("osb_deconv3d_k4_tc_cs_fwd", x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), yp, b, cin, cout, d, h, w, act, ctot,
+        _call("osb_deconv3d_k4_tc_cs" + sfx, x_ndhwc.data_ptr(), wptr, _ptr(scale), _ptr(shift), yp, b, cin, cout, d, h, w, act, ctot,
               _stream(y))
     return y
 
@@ -695,13 +773,16 @@ def feature_att_gate(feat, w1, scale1, shift1, w2, scale2, shift2, pad_to=None, 
 
 def conv1x1_ndhwc_cat(x0, x1, w_packed, scale=None, shift=None, act=ACT_NONE):
     """Channels-last 1x1x1 conv over torch.cat((x0, x1), -1) without materialising it: (..., C0), (..., C1) -> (..., Cout);
-    w_packed (C0 + C1, Cout)."""
-    assert x0.is_cuda and x0.dtype == torch.float32 and x0.is_contiguous() and x1.is_contiguous() and x0.shape[:-1] == x1.shape[:-1]
+    w_packed (C0 + C1, Cout).  fp16 x0 and x1: fp16 output, fp32 weights and arithmetic."""
+    assert x0.is_cuda and x0.is_contiguous() and x1.is_contiguous() and x0.shape[:-1] == x1.shape[:-1]
+    h16 = _is_h16(x0, what="x0")
+    if x1.dtype != x0.dtype:
+        raise ValueError("conv1x1_ndhwc_cat: x0 is %s but x1 is %s" % (x0.dtype, x1.dtype))
     c0, c1 = x0.shape[-1], x1.shape[-1]
     cin, cout = w_packed.shape
-    assert cin == c0 + c1 and w_packed.is_contiguous()
-    y = torch.empty(x0.shape[:-1] + (cout,), dtype=torch.float32, device=x0.device)
-    _call("osb_conv1x1_ndhwc_cat_fwd", x0.data_ptr(), x1.data_ptr(), c0, c1, w_packed.data_ptr(), _ptr(scale), _ptr(shift),
+    assert cin == c0 + c1 and w_packed.is_contiguous() and w_packed.dtype == torch.float32
+    y = torch.empty(x0.shape[:-1] + (cout,), dtype=x0.dtype, device=x0.device)
+    _call("osb_conv1x1_ndhwc_cat_h16_fwd" if h16 else "osb_conv1x1_ndhwc_cat_fwd", x0.data_ptr(), x1.data_ptr(), c0, c1, w_packed.data_ptr(), _ptr(scale), _ptr(shift),
           y.data_ptr(), x0.numel() // c0, cout, act, _stream(y))
     return y
 

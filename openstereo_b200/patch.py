@@ -209,11 +209,11 @@ def _rebind_methods(model, overrides):
             setattr(model, name, types.MethodType(copy, model))
 
 
-def _patch_stereobase(model, strict, backbone=True):
+def _patch_stereobase(model, strict, backbone=True, precision="fp32"):
     g = type(model).forward.__globals__                             # stereo.modeling.models.stereobase.stereobase_gru namespace
     hg = model.cost_agg
     hg_orig = hg.forward
-    agg = StereoBaseAggregation(hg)
+    agg = StereoBaseAggregation(hg, precision=precision)
     orig = {n: g[n] for n in ("build_gwc_volume", "build_concat_volume", "disparity_regression", "CombinedGeoEncodingVolume",
                               "context_upsample")}
 
@@ -333,17 +333,32 @@ _PATCHERS = {"GwcNet": _patch_gwcnet, "PSMNet": _patch_psmnet, "StereoBase": _pa
              "IGEVStereo": _patch_igev}
 
 
-def patch(model, strict=True, backbone=True):
+def patch(model, strict=True, backbone=True, precision="fp32"):
     """Rebind the hot path of a reference model instance in place and return it.  backbone=True (default) also routes the
     GwcNet / PSMNet 2D extractor's residual blocks to the tcgen05 conv kernels in CUDA inference calls (_patch_backbone);
-    backbone=False leaves the extractor entirely to the reference's cuDNN code."""
+    backbone=False leaves the extractor entirely to the reference's cuDNN code.
+
+    precision="fp32" (default): every accelerated op computes fp32-accurate results, also under torch.autocast (fp16 / bf16
+    tensors are up-converted and the results cast back).  precision="fp16" (StereoBase only): under torch.autocast(float16) the
+    cost-aggregation hourglass runs with fp16 activations and one fp16 tensor-core product per multiply-add (fp32 accumulation,
+    BN / activation / FeatureAtt gate in fp32) and returns fp16 -- an accuracy choice like allow_tf32, not a free speed-up.  Its
+    envelope is fp16's: intermediate values are stored as fp16, so |values| above 65504 saturate; when that happens the next
+    forward raises RuntimeError (the saturated result was already returned).  Volumes, classifier head and regression keep fp32
+    arithmetic; fp32 and bf16 inputs and shapes without the fp16 kernels take the fp32 path (INTEGRATION.md section 1)."""
     if not isinstance(model, torch.nn.Module):
         raise TypeError("patch() expects an nn.Module")
+    if precision not in ("fp32", "fp16"):
+        raise ValueError("precision must be 'fp32' or 'fp16', got %r" % (precision,))
     name = type(model).__name__
+    if precision == "fp16" and name != "StereoBase":
+        raise ValueError("precision='fp16' is implemented for StereoBase only")
     if name not in _PATCHERS:
         raise NotImplementedError("patch(): no hot-path drop-in for %s (supported: %s)" % (name, sorted(_PATCHERS)))
     if getattr(model, "_osb_patched", False):
         return model
-    _PATCHERS[name](model, strict, backbone)
+    if precision == "fp16":
+        _PATCHERS[name](model, strict, backbone, precision=precision)
+    else:
+        _PATCHERS[name](model, strict, backbone)
     model._osb_patched = True
     return model

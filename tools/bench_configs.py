@@ -1,12 +1,16 @@
 #!/usr/bin/env python
 """Hot-path timings at the OTHER BASELINE.json configurations (bench.py is the contract line for configs[1], GwcNet):
 
-    python tools/bench_configs.py [--only c1,c3,c4,c5] [--iters 10]
+    python tools/bench_configs.py [--only c1,c3,c3h,c4,c5] [--iters 10]
 
   c1  PSMNet cfgs/psmnet, 1 pair 256x512 D=192: whole-model forward of the host mirror (pairs/s) + EPE vs the CPU oracle
   c3  StereoBase cfgs/stereobase, 4 pairs/GPU (batch 32 over 8 GPUs) @256x512: the hot sub-graph on synthetic features --
       gwc (C=96, G=8) + concat (C=8) volume -> Hourglass(24, [96,64,192,160]) with FeatureAtt gates -> classifier -> softmax ->
       regression (stereobase_gru.py:139-164)
+  c3h the c3 sub-graph under torch.autocast("cuda", torch.float16), as StereoBase's own AMP configs evaluate it
+      (stereobase_sceneflow.yaml AMP: true): three arms alternated in one process -- (a) the oracle modules on cuDNN fp16 (the
+      reference's AMP behaviour), (b) this library with precision="fp32" (fp32-accurate hourglass), (c) precision="fp16" (fp16
+      hourglass) -- with per-kernel times of (b) and (c) and the init-disparity EPE of (a) and (c) against (b)
   c4  LightStereo-S cfgs/lightstereo, batch 16 @320x736: correlation_volume (C=24... the 1/4 features) -> Aggregation(48, [1,2,4],
       expanse 4, left attention) -> softmax/regression -> context_upsample (lightstereo.py:51-62)
   c5  IGEV cfgs/igev, batch 8 @480x640: gwc volume (C=96, G=8, D'=48) + 16 GRU-iteration lookups of the combined geometry
@@ -135,6 +139,72 @@ def c3(iters, B=4):
          gmac_per_pair=23.48)
 
 
+def gpu_identity():
+    """(name, power limit) of the GPU these numbers were measured on, read in the same process."""
+    import subprocess
+    try:
+        q = subprocess.run(["nvidia-smi", "-i", str(DEV.index), "--query-gpu=power.limit,clocks.max.sm", "--format=csv,noheader"],
+                           capture_output=True, text=True, timeout=30).stdout.strip()
+    except (OSError, subprocess.SubprocessError) as exc:
+        q = "unavailable (%s)" % exc
+    return torch.cuda.get_device_name(DEV), q
+
+
+def c3h(iters, B=4, rounds=5):
+    gen = torch.Generator().manual_seed(7)
+    ml, mr, cl, cr = (rnd(gen, B, 96, 64, 128).half(), rnd(gen, B, 96, 64, 128).half(), rnd(gen, B, 8, 64, 128).half(),
+                      rnd(gen, B, 8, 64, 128).half())
+    feats = [rnd(gen, B, 96, 64, 128).half(), rnd(gen, B, 64, 32, 64).half(), rnd(gen, B, 192, 16, 32).half(),
+             rnd(gen, B, 160, 8, 16).half()]
+    m = oagg.StereoBaseCostHead(24, [96, 64, 192, 160], max_disp=192).eval()
+    m.load_state_dict(si.seeded_state_dict(m.state_dict(), seed=9, scale={"classifier.weight": 150.0}))
+    m.to(DEV)
+    head = agg.StereoBaseCostHead(m.classifier)
+    engines = {"fp32": agg.StereoBaseAggregation(m.cost_agg), "fp16": agg.StereoBaseAggregation(m.cost_agg, precision="fp16")}
+
+    def ours(precision):
+        def step():   # patch.py's StereoBase route: fp16 volume in, the hourglass result cast back to the volume's dtype
+            vol = ops.gwc_concat_volume(ml, mr, cl, cr, 48, 8)
+            return head(engines[precision](vol, feats).to(vol.dtype), 48)
+        return step
+
+    def ref():
+        vol = torch.cat((ocv.build_gwc_volume(ml, mr, 48, 8), ocv.build_concat_volume(cl, cr, 48)), 1)
+        return m(vol, feats)[1]
+
+    arms = {"a_reference_cudnn_fp16": ref, "b_ours_fp32": ours("fp32"), "c_ours_fp16": ours("fp16")}
+    times = {k: [] for k in arms}
+    outs = {}
+    with torch.no_grad(), torch.autocast("cuda", torch.float16):
+        for k, fn in arms.items():                                          # warm every arm (module loads, cuDNN algorithm choice)
+            outs[k] = fn().float()
+        for _ in range(rounds):                                             # alternate the arms: drift of the shared host hits all
+            for k, fn in arms.items():
+                ms, _ = timeit(fn, iters, warm=1)
+                times[k].append(ms)
+        kernels = {}
+        for k in ("b_ours_fp32", "c_ours_fp16"):                            # per entry point, CUDA events (separate from the timing)
+            arms[k]()
+            torch.cuda.synchronize()
+            ops.profile_start()
+            for _ in range(iters):
+                arms[k]()
+            prof = ops.profile_stop()
+            torch.cuda.synchronize()
+            kernels[k] = {n: round(sum(a.elapsed_time(b) for a, b in ev) / iters, 4) for n, ev in sorted(prof.items())}
+    med = {k: sorted(v)[len(v) // 2] for k, v in times.items()}
+    name, power = gpu_identity()
+    base = outs["b_ours_fp32"]
+    emit(config="c3h StereoBase hot sub-graph under autocast(fp16), B=%d @256x512" % B, gpu=name, power_limit_and_max_sm_clock=power,
+         iters_per_round=iters, rounds=rounds, ms_per_step_median={k: round(v, 3) for k, v in med.items()},
+         ms_per_step_all={k: [round(x, 3) for x in v] for k, v in times.items()},
+         speedup_c_vs_b=round(med["b_ours_fp32"] / med["c_ours_fp16"], 3),
+         speedup_c_vs_a=round(med["a_reference_cudnn_fp16"] / med["c_ours_fp16"], 3),
+         init_disp_epe_vs_b_px={"a_reference_cudnn_fp16": float("%.3e" % (outs["a_reference_cudnn_fp16"] - base).abs().mean().item()),
+                                "c_ours_fp16": float("%.3e" % (outs["c_ours_fp16"] - base).abs().mean().item())},
+         per_entry_point_ms_per_step=kernels, overflow_count=ops.tc_overflow_count())
+
+
 def c4(iters, B=16):
     gen = torch.Generator().manual_seed(11)
     h, w = 80, 184
@@ -247,12 +317,12 @@ def gw(iters):
 
 if __name__ == "__main__":
     ap = argparse.ArgumentParser()
-    ap.add_argument("--only", default="c1,c3,c4,c5,gw")
+    ap.add_argument("--only", default="c1,c3,c3h,c4,c5,gw")
     ap.add_argument("--iters", type=int, default=10)
     a = ap.parse_args()
     for name in a.only.split(","):
         try:
-            {"c1": c1, "c3": c3, "c4": c4, "c5": c5, "gw": gw}[name](a.iters)
+            {"c1": c1, "c3": c3, "c3h": c3h, "c4": c4, "c5": c5, "gw": gw}[name](a.iters)
         except Exception as exc:                                               # one config must not hide the others
             emit(config=name, error=repr(exc)[:300])
     if WORLD > 1:
